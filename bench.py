@@ -36,8 +36,8 @@ BYTES_PER_POINT = 16
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, help="timed steps (default 20)")
+    ap.add_argument("--warmup", type=int, help="warm-up steps (default 3)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--lanes", type=int, default=int(os.environ.get("LIODOM_BENCH_LANES", "128")),
                     help="independent sequences per GPU processed by one step")
@@ -55,7 +55,18 @@ def parse():
     ap.add_argument("--no-stage-pass", action="store_true")
     ap.add_argument("--no-single-stream", action="store_true")
     ap.add_argument("--no-xyz12", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0's lanes) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.config == "c4" and (args.steps is not None or args.warmup is not None):
+        ap.error("--config c4 times --frames map updates after one warm-up frame; it takes no --steps / --warmup")
+    args.steps = 20 if args.steps is None else args.steps
+    args.warmup = 3 if args.warmup is None else args.warmup
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config == "c4" or args.mode != "sequences"):
+        ap.error("--dump-outputs applies to the default path (--impl b200 --mode sequences, config c1 / c2 / c3)")
+    return args
 
 
 def dist_env():
@@ -268,6 +279,8 @@ def run_b200(args):
     launches = ctx.launch_count - launches0
     poses_dev, nedges = ctx.results()
     value = world * B * K / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, poses_dev, nedges)
 
     # ---------------- per-stage pass (roofline of the dominant kernel) ----------------------
     roof = None
@@ -563,6 +576,24 @@ def run_b200(args):
     if cpu is not None:
         out["cpu_baseline"] = cpu
     emit(out)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ctx, poses, nedges):
+    """What a caller of the device-resident path receives for the last timed step, so that two builds can be
+    compared output for output on the same seeded inputs: poses [lanes,4,4] (f64), edge counts [lanes] (as f64) and
+    the edge clouds of all lanes back to back [sum(edges),4] (f32 x, y, z, intensity).  Edge rows beyond the 64 MB
+    budget are thinned to a fixed seeded sample (the same rows whenever the edge counts agree)."""
+    os.makedirs(out_dir, exist_ok=True)
+    edges = np.concatenate([ctx.scan_edges(l) for l in range(ctx.batch)])
+    room = max((DUMP_BYTES - poses.nbytes - 8 * nedges.size) // (edges.itemsize * edges.shape[1]), 0)
+    if len(edges) > room:
+        edges = edges[np.sort(np.random.default_rng(0).choice(len(edges), room, replace=False))]
+    np.save(os.path.join(out_dir, "poses.npy"), np.asarray(poses, np.float64))
+    np.save(os.path.join(out_dir, "n_edges.npy"), np.asarray(nedges, np.float64))
+    np.save(os.path.join(out_dir, "edges.npy"), np.asarray(edges, np.float32))
 
 
 def single_stream_block(api, torch, dev, local, scans, npts, kw, P, W, K, width, height):

@@ -16,7 +16,7 @@ import oracle
 from oracle import ref
 from conftest import get_sequence, pose_err
 
-pytestmark = pytest.mark.skipif(not ref.dropin_available(), reason="drop-in libraries not built and /root/reference absent")
+pytestmark = pytest.mark.skipif(not ref.dropin_available(), reason="needs the upstream liodom sources (LIODOM_REFERENCE_ROOT) or a prebuilt oracle/_ref")
 
 
 def _pose_from_odom(row):

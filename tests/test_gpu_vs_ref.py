@@ -8,7 +8,7 @@ from oracle import ref
 from liodom_b200 import api
 from conftest import get_sequence, pose_err
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built")]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref.available(), reason="needs the upstream liodom sources (LIODOM_REFERENCE_ROOT) or a prebuilt oracle/_ref")]
 
 
 def _bits(a):

@@ -24,7 +24,7 @@ import oracle
 from oracle import ref
 from conftest import get_sequence, pose_err
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built and /root/reference absent")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="needs the upstream liodom sources (LIODOM_REFERENCE_ROOT) or a prebuilt oracle/_ref")
 
 
 def _bits(a):
