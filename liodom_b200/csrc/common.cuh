@@ -242,6 +242,9 @@ __device__ __forceinline__ unsigned hash_cell(unsigned long long k) {
   k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
   return (unsigned)k;
 }
+// Edge-sharded mode (world > 1 ranks per lane): rank r associates and solves the Morton positions
+// [r * share, (r + 1) * share) of the lane's n edges.  A multiple of 32, so every rank starts on a warp boundary.
+__host__ __device__ __forceinline__ int edge_share(int n, int world) { return ((n + world - 1) / world + 31) & ~31; }
 // word of the occupancy filter holding cell (ix, iy, iz): 32 consecutive cells along x share a word
 __device__ __forceinline__ unsigned bloom_word_index(int ixhi, int iy, int iz, unsigned bmask) {
   unsigned h = (unsigned)ixhi * 0x9E3779B1u ^ (unsigned)iy * 0x85EBCA77u ^ (unsigned)iz * 0xC2B2AE3Du;

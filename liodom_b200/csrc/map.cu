@@ -641,7 +641,6 @@ int liodom_map_create(double voxel_xysize, double voxel_zsize, double resolution
     MCC(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     if (per_sm < 1) { mfail(nullptr, LIODOM_E_CUDA, "k_map_update cannot be made resident"); liodom_map_destroy(c); return LIODOM_E_CUDA; }
     c->coop_blocks = sms;   // one CTA per SM: the phases are short, more CTAs only lengthen the grid barriers
-    if (const char* e = getenv("LIODOM_MAP_BLOCKS")) { const int v = atoi(e); if (v >= 1 && v <= sms * per_sm) c->coop_blocks = v; }
   }
   MCC(cudaStreamSynchronize(c->stream));
 #undef MCC

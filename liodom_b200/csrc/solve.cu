@@ -463,7 +463,7 @@ __global__ void __launch_bounds__(kShardThreads) k_shard_step(DevBuffers d, int 
     double xs[7];
     for (int k = 0; k < 7; ++k) xs[k] = action == 0 ? c.x[k] : c.xc[k];
     const int E = os.n_edges;
-    const int share = ((E + world - 1) / world + 31) & ~31;     // same partition as k_associate
+    const int share = edge_share(E, world);
     const int t1 = min(E, (rank + 1) * share);
     const float* blocks = d.blocks + (size_t)lane_b * p.Ecap * 10;
     const int* perm = d.perm + (size_t)lane_b * p.Ecap;

@@ -88,15 +88,6 @@ def test_batch128_lane_groups(cuda_lib, groups, monkeypatch):
     print("batch 128, %s lane groups: worst pose error %.3g m %.3g rad" % (groups, w[0], w[1]))
 
 
-def test_batch128_cta_level_association(cuda_lib, monkeypatch):
-    """LIODOM_ASSOC_CTA=1: the CTA-level, work-balanced association kernel (k_associate_cta: edges sorted by bucket
-    length in shared memory, listed neighbour buckets, flattened scan) must give the same neighbours, hence the same
-    poses, as the thread-per-edge kernel.  Its teacher-forced bit-exactness runs in test_gpu_register.py."""
-    monkeypatch.setenv("LIODOM_ASSOC_CTA", "1")
-    w = _run_batch(128, "device")
-    print("batch 128, CTA-level association: worst pose error %.3g m %.3g rad" % (w[0], w[1]))
-
-
 @pytest.mark.parametrize("pool", ["0", "1"])
 def test_batch128_warp_pooled_association(cuda_lib, pool, monkeypatch):
     """LIODOM_ASSOC_POOL=0 / 1: the thread-per-edge kernel in both outer iterations / the warp-pooled one in both (the

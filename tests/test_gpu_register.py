@@ -81,16 +81,12 @@ def _teacher_forced_associate(ctx, edges_seq, gt, K):
     return nchecked
 
 
-@pytest.mark.parametrize("group", ["1", "4", "8", "16", "cta", "pool", "thread"])
+@pytest.mark.parametrize("group", ["1", "4", "8", "16", "pool", "thread"])
 def test_associate_teacher_forced_c1(cuda_lib, group, monkeypatch):
-    """Every kernel variant (1, 4, 8 or 16 threads per edge; picked by the number of edges in flight), the warp-pooled
-    form of the one-thread-per-edge search (LIODOM_ASSOC_POOL=1 / 0) and the opt-in CTA-level one (LIODOM_ASSOC_CTA=1)."""
-    monkeypatch.delenv("LIODOM_ASSOC_CTA", raising=False)
+    """Every kernel variant (1, 4, 8 or 16 threads per edge; picked by the number of edges in flight) and the warp-pooled
+    form of the one-thread-per-edge search (LIODOM_ASSOC_POOL=1 / 0)."""
     monkeypatch.delenv("LIODOM_ASSOC_POOL", raising=False)
-    if group == "cta":
-        monkeypatch.setenv("LIODOM_ASSOC_CTA", "1")
-        group = "1"
-    elif group in ("pool", "thread"):
+    if group in ("pool", "thread"):
         monkeypatch.setenv("LIODOM_ASSOC_POOL", "1" if group == "pool" else "0")
         group = "1"
     monkeypatch.setenv("LIODOM_ASSOC_GROUP", group)

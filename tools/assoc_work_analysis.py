@@ -2,7 +2,7 @@
 """Offline replay of the association's work distribution on C1 data (CPU only, oracle + NumPy): per query the points in its
 own 0.5 m cell, in the 27-cell cube, and in the cells that survive the bound of the own cell / the final bound; and how
 well 32 consecutive queries balance under different orderings (Morton, own-cell population, exact work).  The numbers
-quoted in DESIGN.md §5 and in k_associate_cta's comment come from here.
+quoted in DESIGN.md §5 come from here.
 
     python tools/assoc_work_analysis.py
 """
