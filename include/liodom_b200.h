@@ -178,7 +178,18 @@ int liodom_scan_batch(liodom_ctx* ctx, const void* const* pts, const int* n, int
 /* Same with raw PointCloud2 blobs: data[l] holds height x row_step bytes (n[l] = width * height points). */
 int liodom_scan_batch_layout(liodom_ctx* ctx, const void* const* data, const int* n, const liodom_cloud_layout* layout,
                              int width, int height, int on_device);
-/* poses16_out[batch*16], n_edges_out[batch] (either may be NULL) of the last enqueued scan. */
+/* Step only the listed lanes: lanes[i] takes the scan pts[i] / n[i].  Every other lane's state (pose, window, voxel
+ * hash, received map, IMU inputs) is left bit for bit as it was.  Same staging, asynchrony and two-in-flight rules as
+ * liodom_scan_batch; host scans back to back in list order go over in one copy.  lanes: any order, no duplicates,
+ * each in [0, batch); n_lanes in [0, batch]; n_lanes == 0 enqueues nothing and returns 0.  A bad list returns
+ * LIODOM_E_INVALID and enqueues nothing, as does a point-sharded context (it keeps liodom_scan_batch).  The launches
+ * are those of a batch-n_lanes context. */
+int liodom_scan_lanes(liodom_ctx* ctx, const int32_t* lanes, int n_lanes, const void* const* pts, const int* n,
+                      int stride_bytes, int width, int height, int on_device);
+int liodom_scan_lanes_layout(liodom_ctx* ctx, const int32_t* lanes, int n_lanes, const void* const* data, const int* n,
+                             const liodom_cloud_layout* layout, int width, int height, int on_device);
+/* poses16_out[batch*16], n_edges_out[batch] (either may be NULL) of the last enqueued scan.  A lane that step left
+ * out (liodom_scan_lanes) reports n_edges = -1 and its last reported pose (zeros if it was never stepped). */
 int liodom_scan_results(liodom_ctx* ctx, double* poses16_out, int* n_edges_out);
 /* Same for age 0 (last enqueued) or 1 (the scan before it): with two scans in flight the caller
  * enqueues scan k+1, then collects scan k, so the H2D copy of k+1 overlaps the kernels of k.

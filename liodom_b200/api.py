@@ -294,8 +294,38 @@ class Context:
         ns = (ctypes.c_int * self.batch)(*counts)
         self._ck(self.lib.liodom_scan_batch_layout(self.h, p, ns, ctypes.byref(layout), width, height, 1 if on_device else 0))
 
+    def scan_lanes(self, lanes, scans, width=0, height=0):
+        """Step only lanes[i] with the host scan scans[i] (float32 [n,4] or [n,8]); every other lane stays as it was."""
+        assert len(lanes) == len(scans)
+        arrs = [_pts(s) for s in scans]
+        stride = arrs[0].shape[1] * 4 if arrs else 16
+        self._keep = arrs  # keep alive until results()
+        self._scan_lanes(lanes, [a.ctypes.data for a in arrs], [len(a) for a in arrs], stride, width, height, False)
+
+    def scan_lanes_ptrs(self, lanes, ptrs, counts, stride_bytes, width=0, height=0, on_device=True):
+        """scan_lanes with integer addresses (device when on_device, else pinned/pageable host)."""
+        self._scan_lanes(lanes, ptrs, counts, stride_bytes, width, height, on_device)
+
+    def scan_lanes_layout(self, lanes, blobs, counts, layout, width=0, height=0):
+        """liodom_scan_lanes_layout: blobs[i] is a uint8 host array of raw PointCloud2 data for lanes[i]."""
+        assert len(lanes) == len(blobs) == len(counts)
+        arrs = [np.ascontiguousarray(b, dtype=np.uint8) for b in blobs]
+        k = len(arrs)
+        self._keep = arrs
+        self._ck(self.lib.liodom_scan_lanes_layout(self.h, (ctypes.c_int32 * k)(*lanes), k, (_vp * k)(*[a.ctypes.data for a in arrs]),
+                                                   (ctypes.c_int * k)(*counts), ctypes.byref(layout), width, height, 0))
+
+    def _scan_lanes(self, lanes, ptrs, counts, stride_bytes, width, height, on_device):
+        k = len(lanes)
+        assert len(ptrs) == k and len(counts) == k
+        self._ck(self.lib.liodom_scan_lanes(self.h, (ctypes.c_int32 * k)(*lanes), k, (_vp * k)(*ptrs), (ctypes.c_int * k)(*counts),
+                                            stride_bytes, width, height, 1 if on_device else 0))
+
     def results(self, age=0):
-        """Poses [batch,4,4] and edge counts of the last enqueued scan (age 0) or the one before (age 1)."""
+        """Poses [batch,4,4] and edge counts of the last enqueued scan (age 0) or the one before (age 1).
+
+        After a partial step (scan_lanes) a lane that was not stepped has n_edges == -1; its pose row is its last
+        reported pose (zeros if it was never stepped)."""
         poses = np.empty((self.batch, 16))
         ne = np.empty(self.batch, np.int32)
         self._ck(self.lib.liodom_scan_results_of(self.h, age, _p(poses), _p(ne)))

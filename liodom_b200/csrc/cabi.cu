@@ -30,6 +30,7 @@ struct liodom_ctx {
   // so that the tail of one group's latency-bound kernels (k_associate, k_solve) overlaps another group's work
   static constexpr int kMaxGroups = 8;
   int groups = 1;
+  bool groups_forced = false;   // LIODOM_LANE_GROUPS was set at creation
   cudaStream_t group_stream[kMaxGroups] = {};
   cudaEvent_t ev_fork = nullptr, ev_join[kMaxGroups] = {};
   std::vector<void*> allocs;
@@ -40,8 +41,13 @@ struct liodom_ctx {
   void* dev_in[2] = {nullptr, nullptr};
   size_t dev_in_bytes = 0;      // per buffer
   size_t dev_in_lane_bytes = 0;
+  // Per scan in flight: B lane-indexed descriptors followed by the step's lane list (B ints; liodom_scan_lanes only),
+  // staged in one pinned block and sent in one copy (see scan_batch_impl).  d_scan[0] == d.scan.
   ScanDesc* h_desc[2] = {nullptr, nullptr};   // pinned
-  ScanDesc* d_scan[2] = {nullptr, nullptr};   // device descriptors, one set per scan in flight (d_scan[0] == d.scan)
+  ScanDesc* d_scan[2] = {nullptr, nullptr};
+  // A step that left lanes out (partial) reports n_edges = -1 for the lanes with stepped[buf][l] == 0.
+  bool partial[2] = {false, false};
+  std::vector<uint8_t> stepped[2];
   double* h_poses[2] = {nullptr, nullptr};    // pinned [B*16]
   int* h_nedges[2] = {nullptr, nullptr};      // pinned [B]
   cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
@@ -72,6 +78,13 @@ static void stage_mark(liodom_ctx* c) {
 }
 
 static thread_local std::string g_create_err;
+
+// Descriptor slots of one staging buffer: B descriptors, then room for a list of B lane indices.
+static size_t desc_slots(int B) { return B + (sizeof(int32_t) * B + sizeof(ScanDesc) - 1) / sizeof(ScanDesc); }
+static int32_t* lane_list(ScanDesc* descs, int B) { return reinterpret_cast<int32_t*>(descs + B); }
+
+// Lane groups for a step of n lanes.  Measured at 128 lanes: 2 groups +4 %, 4 groups +0 %; at 32 lanes 2 groups -6 %.
+static int default_lane_groups(int n) { return n >= 64 ? 2 : 1; }
 
 static int fail(liodom_ctx* c, int code, const char* fmt, ...) {
   char buf[512];
@@ -178,8 +191,8 @@ int liodom_ctx_create(const liodom_params* up, int batch, int device, liodom_ctx
   CKC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   c->timeline = getenv("LIODOM_TIMELINE") != nullptr;
   {
-    int g = batch >= 64 ? 2 : 1;   // measured at 128 lanes: 2 groups +4 %, 4 groups +0 %; at 32 lanes 2 groups -6 %
-    if (const char* e = getenv("LIODOM_LANE_GROUPS")) g = atoi(e);
+    int g = default_lane_groups(batch);
+    if (const char* e = getenv("LIODOM_LANE_GROUPS")) { g = atoi(e); c->groups_forced = true; }
     c->groups = std::max(1, std::min(std::min(g, batch), (int)liodom_ctx::kMaxGroups));
     CKC(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
     for (int k = 0; k < c->groups && c->groups > 1; ++k) {
@@ -227,7 +240,7 @@ int liodom_ctx_create(const liodom_params* up, int batch, int device, liodom_ctx
   }
   CKC(configure_extract_kernels());   // per device: a second context on another GPU needs its own opt-in
   const size_t B = batch, L = P.scan_lines;
-  CKC(dalloc(c, &d.scan, B));
+  CKC(dalloc(c, &d.scan, desc_slots(batch)));
   CKC(dalloc(c, &d.ring_id, B * p.Ncap, false));
   CKC(dalloc(c, &d.chunk_hist, B * p.chunks * L));
   CKC(dalloc(c, &d.chunk_base, B * p.chunks * L));
@@ -281,14 +294,15 @@ int liodom_ctx_create(const liodom_params* up, int batch, int device, liodom_ctx
   CKC(dalloc(c, &c->stage_sum, 1));
   CKC(dalloc(c, &c->stage_pose, 12));
   for (int k = 0; k < 2; ++k) {
-    CKC(cudaMallocHost(&c->h_desc[k], sizeof(ScanDesc) * B));
+    CKC(cudaMallocHost(&c->h_desc[k], sizeof(ScanDesc) * desc_slots(batch)));
+    c->stepped[k].assign(B, 0);
     CKC(cudaMallocHost(&c->h_poses[k], sizeof(double) * 16 * B));
     CKC(cudaMallocHost(&c->h_nedges[k], sizeof(int) * B));
     CKC(cudaEventCreateWithFlags(&c->ev_copied[k], cudaEventDisableTiming));
     CKC(cudaEventCreateWithFlags(&c->ev_done[k], cudaEventDisableTiming));
   }
   c->d_scan[0] = d.scan;
-  CKC(dalloc(c, &c->d_scan[1], B));
+  CKC(dalloc(c, &c->d_scan[1], desc_slots(batch)));
   c->dprod = c->d;
   c->dprod.gate = nullptr; c->dprod.knn_idx = nullptr; c->dprod.knn_d2 = nullptr; c->dprod.eig = nullptr;
   c->dprod.q_world = nullptr; c->dprod.src_index = nullptr;
@@ -777,61 +791,102 @@ int liodom_register(liodom_ctx* c, int lane, const float* edges_xyzi, int n_edge
 }
 
 // ---- whole hot path, batched --------------------------------------------------------------
-static int scan_batch_impl(liodom_ctx* c, const void* const* pts, const int* n, const Layout& lay, int width, int height, int on_device);
+// lanes == nullptr: every lane, position l = lane l (liodom_scan_batch).  Otherwise position i steps lane lanes[i].
+static int scan_batch_impl(liodom_ctx* c, const int32_t* lanes, int n_lanes, const void* const* pts, const int* n, const Layout& lay,
+                           int width, int height, int on_device);
 
 int liodom_scan_batch(liodom_ctx* c, const void* const* pts, const int* n, int stride_bytes, int width, int height, int on_device) {
   if (!c) return LIODOM_E_INVALID;
   Layout lay;
   int rc = layout_from_stride(c, stride_bytes, &lay); if (rc) return rc;
-  return scan_batch_impl(c, pts, n, lay, width, height, on_device);
+  return scan_batch_impl(c, nullptr, c->batch, pts, n, lay, width, height, on_device);
 }
 
 int liodom_scan_batch_layout(liodom_ctx* c, const void* const* data, const int* n, const liodom_cloud_layout* layout, int width, int height, int on_device) {
   if (!c) return LIODOM_E_INVALID;
   Layout lay;
   int rc = layout_from_user(c, layout, width, &lay); if (rc) return rc;
-  return scan_batch_impl(c, data, n, lay, width, height, on_device);
+  return scan_batch_impl(c, nullptr, c->batch, data, n, lay, width, height, on_device);
 }
 
-static int scan_batch_impl(liodom_ctx* c, const void* const* pts, const int* n, const Layout& lay, int width, int height, int on_device) {
+// A lane list from the caller: in range, no duplicates, not on a point-sharded context.
+static int check_lane_list(liodom_ctx* c, const int32_t* lanes, int n_lanes, const void* const* pts, const int* n) {
+  if (c->shard.world > 1) return fail(c, LIODOM_E_INVALID, "a point-sharded context steps its one lane with liodom_scan_batch");
+  if (n_lanes < 0 || n_lanes > c->batch) return fail(c, LIODOM_E_INVALID, "n_lanes %d outside [0,%d]", n_lanes, c->batch);
+  if (n_lanes > 0 && (!lanes || !pts || !n)) return fail(c, LIODOM_E_INVALID, "lanes, pts and n must not be NULL");
+  std::vector<uint8_t> seen(c->batch, 0);
+  for (int i = 0; i < n_lanes; ++i) {
+    const int l = lanes[i];
+    if (l < 0 || l >= c->batch) return fail(c, LIODOM_E_INVALID, "lanes[%d] = %d outside [0,%d)", i, l, c->batch);
+    if (seen[l]) return fail(c, LIODOM_E_INVALID, "lane %d listed twice", l);
+    seen[l] = 1;
+  }
+  return 0;
+}
+
+int liodom_scan_lanes(liodom_ctx* c, const int32_t* lanes, int n_lanes, const void* const* pts, const int* n, int stride_bytes,
+                      int width, int height, int on_device) {
+  if (!c) return LIODOM_E_INVALID;
+  int rc = check_lane_list(c, lanes, n_lanes, pts, n); if (rc) return rc;
+  Layout lay;
+  rc = layout_from_stride(c, stride_bytes, &lay); if (rc) return rc;
+  return scan_batch_impl(c, lanes, n_lanes, pts, n, lay, width, height, on_device);
+}
+
+int liodom_scan_lanes_layout(liodom_ctx* c, const int32_t* lanes, int n_lanes, const void* const* data, const int* n,
+                             const liodom_cloud_layout* layout, int width, int height, int on_device) {
+  if (!c) return LIODOM_E_INVALID;
+  int rc = check_lane_list(c, lanes, n_lanes, data, n); if (rc) return rc;
+  Layout lay;
+  rc = layout_from_user(c, layout, width, &lay); if (rc) return rc;
+  return scan_batch_impl(c, lanes, n_lanes, data, n, lay, width, height, on_device);
+}
+
+static int scan_batch_impl(liodom_ctx* c, const int32_t* lanes, int n_lanes, const void* const* pts, const int* n, const Layout& lay,
+                           int width, int height, int on_device) {
   CK(cudaSetDevice(c->device));
+  if (n_lanes == 0) return 0;
   const int B = c->batch;
+  auto lane_of = [&](int i) { return lanes ? (int)lanes[i] : i; };
   int rc;
-  for (int l = 0; l < B; ++l) { rc = check_scan_shape(c, l, n[l], lay, width, height); if (rc) return rc; }
+  for (int i = 0; i < n_lanes; ++i) { rc = check_scan_shape(c, lane_of(i), n[i], lay, width, height); if (rc) return rc; }
   rc = hash_generation_guard(c, 1); if (rc) return rc;
   const int buf = c->cur ^ 1;
   if (c->in_flight[buf]) { CK(cudaEventSynchronize(c->ev_done[buf])); c->in_flight[buf] = false; }
   ScanDesc* hd = c->h_desc[buf];
+  // Descriptors stay lane-indexed (only the listed lanes' are rewritten); the list rides in the same copy.
+  if (lanes) std::memcpy(lane_list(hd, B), lanes, sizeof(int32_t) * n_lanes);
+  const size_t desc_bytes = sizeof(ScanDesc) * B + (lanes ? sizeof(int32_t) * n_lanes : 0);
   if (!on_device) {
     size_t max_bytes = (size_t)c->d.p.Ncap * 32;
-    for (int l = 0; l < B; ++l) max_bytes = std::max(max_bytes, scan_bytes(lay, n[l], width, height));
+    for (int i = 0; i < n_lanes; ++i) max_bytes = std::max(max_bytes, scan_bytes(lay, n[i], width, height));
     rc = ensure_dev_in(c, max_bytes); if (rc) return rc;
-    // Host scans laid out back to back (a batching front-end would do that) go over PCIe as ONE copy
-    // into a packed staging area; otherwise one copy per lane into fixed-pitch slots.
-    bool packed = B > 1 && (lay.step & 3) == 0 && !lay.row_step;   // 4-byte aligned records (16-byte xyzi, 32-byte PCL, 12-byte xyz)
+    // Host scans laid out back to back in list order (a batching front-end would do that) go over PCIe as ONE copy
+    // into a packed staging area; otherwise one copy per list position into fixed-pitch slots.
+    bool packed = n_lanes > 1 && (lay.step & 3) == 0 && !lay.row_step;   // 4-byte aligned records (16-byte xyzi, 32-byte PCL, 12-byte xyz)
     size_t total = 0;
-    for (int l = 0; l < B && packed; ++l) {
-      if (static_cast<const char*>(pts[l]) != static_cast<const char*>(pts[0]) + total) packed = false;
-      total += (size_t)n[l] * lay.step;
+    for (int i = 0; i < n_lanes && packed; ++i) {
+      if (static_cast<const char*>(pts[i]) != static_cast<const char*>(pts[0]) + total) packed = false;
+      total += (size_t)n[i] * lay.step;
     }
     packed = packed && total <= c->dev_in_bytes;
     size_t off = 0;
-    for (int l = 0; l < B; ++l) {
-      char* dst = packed ? static_cast<char*>(c->dev_in[buf]) + off : static_cast<char*>(c->dev_in[buf]) + (size_t)l * c->dev_in_lane_bytes;
-      fill_desc(&hd[l], dst, n[l], lay, width, height);
-      off += (size_t)n[l] * lay.step;
+    for (int i = 0; i < n_lanes; ++i) {
+      char* dst = packed ? static_cast<char*>(c->dev_in[buf]) + off : static_cast<char*>(c->dev_in[buf]) + (size_t)i * c->dev_in_lane_bytes;
+      fill_desc(&hd[lane_of(i)], dst, n[i], lay, width, height);
+      off += (size_t)n[i] * lay.step;
     }
     // The descriptors go FIRST and on the copy stream: a small H2D copy issued on the compute stream would
     // queue behind the next scan's bulk copy on the same copy engine and stall this scan's kernels for
     // the whole transfer (measured: 6.6 ms instead of 2.7 ms of compute per second step at 128 lanes).
-    CK(cudaMemcpyAsync(c->d_scan[buf], hd, sizeof(ScanDesc) * B, cudaMemcpyHostToDevice, c->copy_stream));
+    CK(cudaMemcpyAsync(c->d_scan[buf], hd, desc_bytes, cudaMemcpyHostToDevice, c->copy_stream));
     if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->copy_stream); c->tl_events.push_back(e); }
     if (packed) {
       if (total > 0) CK(cudaMemcpyAsync(c->dev_in[buf], pts[0], total, cudaMemcpyHostToDevice, c->copy_stream));
     } else {
-      for (int l = 0; l < B; ++l) {
-        const size_t bytes = scan_bytes(lay, n[l], width, height);
-        if (bytes > 0) CK(cudaMemcpyAsync(const_cast<void*>(hd[l].pts), pts[l], bytes, cudaMemcpyHostToDevice, c->copy_stream));
+      for (int i = 0; i < n_lanes; ++i) {
+        const size_t bytes = scan_bytes(lay, n[i], width, height);
+        if (bytes > 0) CK(cudaMemcpyAsync(const_cast<void*>(hd[lane_of(i)].pts), pts[i], bytes, cudaMemcpyHostToDevice, c->copy_stream));
       }
     }
     if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->copy_stream); c->tl_events.push_back(e); }
@@ -839,24 +894,26 @@ static int scan_batch_impl(liodom_ctx* c, const void* const* pts, const int* n, 
     CK(cudaStreamWaitEvent(c->stream, c->ev_copied[buf], 0));
     if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->stream); c->tl_events.push_back(e); }
   } else {
-    for (int l = 0; l < B; ++l) fill_desc(&hd[l], pts[l], n[l], lay, width, height);
-    CK(cudaMemcpyAsync(c->d_scan[buf], hd, sizeof(ScanDesc) * B, cudaMemcpyHostToDevice, c->stream));
+    for (int i = 0; i < n_lanes; ++i) fill_desc(&hd[lane_of(i)], pts[i], n[i], lay, width, height);
+    CK(cudaMemcpyAsync(c->d_scan[buf], hd, desc_bytes, cudaMemcpyHostToDevice, c->stream));
   }
   DevBuffers d = c->dprod;
   d.scan = c->d_scan[buf];
-  const LaneRange lr{0, B};
+  d.lanes = lanes ? lane_list(c->d_scan[buf], B) : nullptr;
+  const LaneRange lr{0, n_lanes};
+  // the lane groups a context of n_lanes lanes would use, at most the streams this one has
+  const int G = std::min(std::min(c->groups, n_lanes), c->groups_forced ? c->groups : default_lane_groups(n_lanes));
   int k = 0;
   if (c->shard.world > 1) {
     rc = enqueue_scan_sharded(c, d, &k);
     if (rc) return rc;
-  } else if (c->groups > 1 && !c->stage_timing) {
-    const int G = c->groups;
+  } else if (G > 1 && !c->stage_timing) {
     // fork: every group's chain waits for the descriptors (and the H2D copy) on the main stream
     CK(cudaEventRecord(c->ev_fork, c->stream));
     for (int g = 0; g < G; ++g) CK(cudaStreamWaitEvent(c->group_stream[g], c->ev_fork, 0));
     for (int st = 0; st < 7; ++st)
       for (int g = 0; g < G; ++g) {
-        const int l0 = (int)((long long)B * g / G), l1 = (int)((long long)B * (g + 1) / G);
+        const int l0 = (int)((long long)n_lanes * g / G), l1 = (int)((long long)n_lanes * (g + 1) / G);
         const LaneRange gr{l0, l1 - l0};
         cudaStream_t s = c->group_stream[g];
         {
@@ -891,6 +948,11 @@ static int scan_batch_impl(liodom_ctx* c, const void* const* pts, const int* n, 
   if (c->timeline && !on_device) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->stream); c->tl_events.push_back(e); }
   c->in_flight[buf] = true;
   c->cur = buf;
+  c->partial[buf] = n_lanes < B;
+  if (c->partial[buf]) {
+    std::fill(c->stepped[buf].begin(), c->stepped[buf].end(), 0);
+    for (int i = 0; i < n_lanes; ++i) c->stepped[buf][lanes[i]] = 1;
+  }
   return 0;
 }
 
@@ -928,7 +990,11 @@ int liodom_scan_results_of(liodom_ctx* c, int age, double* poses16_out, int* n_e
   const int buf = c->cur ^ age;
   if (c->in_flight[buf]) { CK(cudaEventSynchronize(c->ev_done[buf])); c->in_flight[buf] = false; }
   if (poses16_out) std::memcpy(poses16_out, c->h_poses[buf], sizeof(double) * 16 * c->batch);
-  if (n_edges_out) std::memcpy(n_edges_out, c->h_nedges[buf], sizeof(int) * c->batch);
+  if (n_edges_out) {
+    std::memcpy(n_edges_out, c->h_nedges[buf], sizeof(int) * c->batch);
+    if (c->partial[buf])
+      for (int l = 0; l < c->batch; ++l) if (!c->stepped[buf][l]) n_edges_out[l] = -1;
+  }
   return 0;
 }
 

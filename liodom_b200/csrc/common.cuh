@@ -187,10 +187,15 @@ struct DevBuffers {
   double* shard_acc;       // [B][32] partial / reduced normal equations of the point-sharded solve
   FrameDiagDev* diag;      // [B]
   double* poses_out;       // [B][16]
+  const int* lanes;        // [n_lanes] lane stepped at each position of a partial step (liodom_scan_lanes); null: identity
 };
 
+// Lane at position `pos` of the step's lane list.
+__device__ __forceinline__ int lane_at(const DevBuffers& d, int pos) { return d.lanes ? d.lanes[pos] : pos; }
+
 // ---- launchers (each returns the number of kernels it enqueued) ----------------------
-// Every kernel works on lanes [lane0, lane0 + nlanes).
+// Every kernel works on the lanes at positions [lane0, lane0 + nlanes) of the step's lane list (lane_at); without a
+// list (d.lanes null, every single-lane entry point) position and lane coincide.
 struct LaneRange { int lane0, nlanes; };
 int launch_split(const DevBuffers& d, cudaStream_t s, LaneRange lr);
 int launch_extract(const DevBuffers& d, cudaStream_t s, LaneRange lr, bool want_keys);

@@ -159,7 +159,7 @@ __device__ __forceinline__ int ring_of_point(const DevParams& p, const ScanDesc&
 // Pass 1: ring id per point + per-chunk histogram. grid (chunks, B), 256 threads, each warp
 // owns a contiguous 256-point segment so that (warp, round, lane) is input order.
 __global__ void __launch_bounds__(256) k_split_count(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y, chunk = blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y), chunk = blockIdx.x;
   const ScanDesc sc = d.scan[lane_b];
   const DevParams& p = d.p;
   const int L = p.scan_lines;
@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(256) k_split_count(DevBuffers d, int lane0) {
 // One thread per ring walks that ring's chunk counts; the loads are issued eight at a time (their addresses do not
 // depend on the running sum), which turns ~60 dependent round trips into ~8 (21 -> 5 us at 128 lanes).
 __global__ void __launch_bounds__(kMaxLines) k_split_scan(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x);
   const DevParams& p = d.p;
   const int L = p.scan_lines, r = threadIdx.x;
   const ScanDesc sc = d.scan[lane_b];
@@ -239,8 +239,8 @@ __global__ void __launch_bounds__(kMaxLines) k_split_scan(DevBuffers d, int lane
 
 // Pass 3: stable scatter into ring-major order. grid (chunks, B), 256 threads.
 __global__ void __launch_bounds__(256) k_split_scatter(DevBuffers d, int lane0) {
-  // CTAs walk the batch in the REVERSE of k_split_count's order: the scans that pass read last are still in L2
-  const int lane_b = lane0 + (int)(gridDim.y - 1u - blockIdx.y), chunk = (int)(gridDim.x - 1u - blockIdx.x);
+  // CTAs walk the lane list in the REVERSE of k_split_count's order: the scans that pass read last are still in L2
+  const int lane_b = lane_at(d, lane0 + (int)(gridDim.y - 1u - blockIdx.y)), chunk = (int)(gridDim.x - 1u - blockIdx.x);
   const ScanDesc sc = d.scan[lane_b];
   const DevParams& p = d.p;
   const int L = p.scan_lines;
@@ -453,7 +453,7 @@ __device__ int run_region_reg(const RingView& rv, const unsigned* gapbits, int w
 template <int NT>
 __global__ void __launch_bounds__(NT, NT == 256 ? 4 : 1) k_extract(DevBuffers d, int lane0, int ring_cap, int want_keys, int ring0) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.y, ring = ring0 + blockIdx.x;   // ring0 > 0: ring-sharded extraction
+  const int lane_b = lane_at(d, lane0 + blockIdx.y), ring = ring0 + blockIdx.x;   // ring0 > 0: ring-sharded extraction
   const int L = p.scan_lines, R = p.scan_regions, epr = p.edges_per_region, E1 = epr + 1;
   const int* roff = d.ring_off + (size_t)lane_b * (L + 1);
   const int off = roff[ring], n = roff[ring + 1] - off;
@@ -634,10 +634,11 @@ __global__ void __launch_bounds__(NT, NT == 256 ? 4 : 1) k_extract(DevBuffers d,
   for (int r = tid; r < R; r += blockDim.x) rcnt[r] = npicks[r];
 }
 
-// Compaction of the fixed slots into the contiguous edge list (ring, region, pick order).
-__global__ void __launch_bounds__(1024) k_compact(DevBuffers d, int lane0) {
+// Compaction of the fixed slots into the contiguous edge list (ring, region, pick order).  Two CTAs per SM (32
+// registers): left free, ptxas spends 42 registers on it once the lane comes from the lane list.
+__global__ void __launch_bounds__(1024, 2) k_compact(DevBuffers d, int lane0) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.x, tid = threadIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x), tid = threadIdx.x;
   const int LR = p.scan_lines * p.scan_regions, E1 = p.edges_per_region + 1;
   extern __shared__ int base[];  // LR + 32
   int* wsum = base + LR;

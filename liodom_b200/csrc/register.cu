@@ -120,7 +120,7 @@ __device__ __forceinline__ void hash_check_generation(const WinState& ws) {
 
 // ---- full, fast ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_hash_insert(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashFullFast) return;
   WinView v;
@@ -150,7 +150,7 @@ __global__ void __launch_bounds__(256) k_hash_insert(DevBuffers d, int lane0) {
 // Bucket allocation: one thread per CELL (the creators appended their slots to owner_list during the insert),
 // a warp-wide prefix of the counts and one bump per warp.
 __global__ void __launch_bounds__(256) k_hash_alloc(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashFullFast) return;
   const int ncell = ws.n_owners, ln = threadIdx.x & 31;
@@ -172,7 +172,7 @@ __global__ void __launch_bounds__(256) k_hash_alloc(DevBuffers d, int lane0) {
 }
 
 __global__ void __launch_bounds__(256) k_hash_scatter(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashFullFast) return;
   WinView v;
@@ -194,8 +194,9 @@ __global__ void __launch_bounds__(256) k_hash_scatter(DevBuffers d, int lane0) {
 // Clears the occupancy filters of the lanes (a kernel, not cudaMemsetAsync: a memset may be placed on a
 // copy engine, where it would wait behind the next scan's H2D transfer).
 __global__ void __launch_bounds__(256) k_bloom_clear(DevBuffers d, int lane0) {
-  if (d.wstate[lane0 + blockIdx.y].hmode != kHashFullFast) return;
-  uint4* w = reinterpret_cast<uint4*>(d.bloom + (size_t)(lane0 + blockIdx.y) * d.p.Bwords);
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
+  if (d.wstate[lane_b].hmode != kHashFullFast) return;
+  uint4* w = reinterpret_cast<uint4*>(d.bloom + (size_t)lane_b * d.p.Bwords);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < d.p.Bwords / 4; i += gridDim.x * blockDim.x) w[i] = make_uint4(0u, 0u, 0u, 0u);
 }
 
@@ -256,7 +257,7 @@ __device__ __forceinline__ void hash_add_count_part(const DevBuffers& d, int lan
 }
 
 __global__ void __launch_bounds__(256) k_hash_evict_add(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   if (d.wstate[lane_b].hmode != kHashIncr) return;
   const int half = gridDim.x >> 1;   // the grid has an even number of CTAs per lane
   if (blockIdx.x & 1) hash_add_count_part(d, lane_b, blockIdx.x >> 1, half);
@@ -268,7 +269,7 @@ __global__ void __launch_bounds__(256) k_hash_evict_add(DevBuffers d, int lane0)
 // heads advance on eviction, tails on insertion — so a steady cell moves once per ~window length of scans.
 constexpr int kGrowGroup = 8;
 __global__ void __launch_bounds__(256) k_hash_grow(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashIncr) return;
   HashEntry* tab = d.htab + (size_t)lane_b * d.p.Hcap;
@@ -299,9 +300,10 @@ __global__ void __launch_bounds__(256) k_hash_grow(DevBuffers d, int lane0) {
   }
 }
 
-// New frame, pass 3: the points go to the tails of their buckets and into the sequence ring.
-__global__ void __launch_bounds__(256) k_hash_add_scatter(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.y;
+// New frame, pass 3: the points go to the tails of their buckets and into the sequence ring.  The bound keeps 8 CTAs
+// per SM (the thread limit): left free, ptxas spends 39 registers on it once the lane comes from the lane list.
+__global__ void __launch_bounds__(256, 8) k_hash_add_scatter(DevBuffers d, int lane0) {
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashIncr) return;
   const unsigned* cell_base = d.cell_base + (size_t)lane_b * d.p.Hcap;
@@ -323,7 +325,7 @@ __global__ void __launch_bounds__(256) k_hash_add_scatter(DevBuffers d, int lane
 // ---- full, ordered: one CTA per lane, frames scattered oldest first so that every bucket is in frame order ----
 constexpr int kFullThreads = 1024;
 __global__ void __launch_bounds__(kFullThreads) k_hash_full_ordered(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x);
   WinState& ws = d.wstate[lane_b];
   if (ws.hmode != kHashFullOrdered) return;
   hash_check_generation(ws);
@@ -512,7 +514,7 @@ __device__ void imu_override(OdomState& os) {
 }
 
 __global__ void k_predict(DevBuffers d, int lane0) {
-  const int lane_b = lane0 + blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x);
   if (threadIdx.x != 0) return;
   OdomState& os = d.ostate[lane_b];
   FrameDiagDev& dg = d.diag[lane_b];
@@ -547,7 +549,7 @@ __device__ __forceinline__ unsigned spread10(unsigned v) {  // 10 bits -> every 
 }
 __global__ void __launch_bounds__(1024) k_edge_order(DevBuffers d, int lane0) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const OdomState& os = d.ostate[lane_b];
   const int base = blockIdx.x * kOrderChunk;
   const int n = min(kOrderChunk, os.n_edges - base);
@@ -958,7 +960,7 @@ template <int G>
 __global__ void __launch_bounds__(kAssocThreads, G == 1 ? kAssocMinBlocks1 : 8) k_associate(DevBuffers d, int lane0, int outer_it, int force,
                                                                              const double* pose_override, int shard_rank, int shard_world) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const OdomState& os = d.ostate[lane_b];
   const bool active = force || os.init;
   const int share = shard_world > 1 ? edge_share(os.n_edges, shard_world) : 0;
@@ -1121,7 +1123,7 @@ __device__ __forceinline__ bool pool_test(const float4& pt, float qx, float qy, 
 __global__ void __launch_bounds__(kAssocThreads, 16) k_associate_pool(DevBuffers d, int lane0, int outer_it, int force,
                                                                                   const double* pose_override, int shard_rank, int shard_world) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const OdomState& os = d.ostate[lane_b];
   const bool active = force || os.init;
   const int share = shard_world > 1 ? edge_share(os.n_edges, shard_world) : 0;
@@ -1288,7 +1290,7 @@ __global__ void __launch_bounds__(kAssocThreads, 16) k_associate_pool(DevBuffers
 // rank's Morton positions).
 __global__ void __launch_bounds__(128) k_line_gate(DevBuffers d, int lane0, int outer_it, int force, int shard_rank, int shard_world) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.y;
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);
   const OdomState& os = d.ostate[lane_b];
   const bool active = force || os.init;
   const int share = shard_world > 1 ? edge_share(os.n_edges, shard_world) : 0;
@@ -1361,7 +1363,7 @@ int launch_associate_shard(const DevBuffers& d, cudaStream_t s, int lane, int ou
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) k_window_update(DevBuffers d, int lane0) {
   const DevParams& p = d.p;
-  const int lane_b = lane0 + blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x);
   OdomState& os = d.ostate[lane_b];
   WinState& ws = d.wstate[lane_b];
   const int E = os.n_edges;
@@ -1382,11 +1384,13 @@ __global__ void __launch_bounds__(1024) k_window_update(DevBuffers d, int lane0)
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    win_commit(d, lane_b, E);
-    hash_begin(d, lane_b);
-    os.init = 1; os.frame++;
-    double* po = d.poses_out + (size_t)lane_b * 16;
-    for (int k = 0; k < 12; ++k) po[k] = os.odom[k];
+    const int lane_c = lane_at(d, lane0 + blockIdx.x);   // looked up again: keeping lane_b across the barrier spills
+    OdomState& os_c = d.ostate[lane_c];
+    win_commit(d, lane_c, E);
+    hash_begin(d, lane_c);
+    os_c.init = 1; os_c.frame++;
+    double* po = d.poses_out + (size_t)lane_c * 16;
+    for (int k = 0; k < 12; ++k) po[k] = os_c.odom[k];
     po[12] = po[13] = po[14] = 0.0; po[15] = 1.0;
   }
 }

@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(kSolveThreads, OCC) k_solve(DevBuffers d, int 
   cg::cluster_group cluster = cg::this_cluster();
   const unsigned C = cluster.num_blocks(), crank = cluster.block_rank();
   const DevParams& p = d.p;
-  const int lane_b = lane0 + (int)(blockIdx.x / C);
+  const int lane_b = lane_at(d, lane0 + (int)(blockIdx.x / C));
   OdomState& os = d.ostate[lane_b];
   if (F32 && !os.init) return;   // uniform over the cluster
   __shared__ LmCtrl c;                                         // authoritative copy lives in CTA 0

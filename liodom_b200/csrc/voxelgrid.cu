@@ -27,7 +27,7 @@ __device__ __forceinline__ bool finite3(const float4& p) { return isfinite(p.x) 
 
 // Lanes whose window is not filtered in this build leave every kernel at once.
 #define VG_LANE_PROLOGUE                                   \
-  const int lane_b = lane0 + blockIdx.y;                   \
+  const int lane_b = lane_at(d, lane0 + blockIdx.y);       \
   WinState& ws = d.wstate[lane_b];                         \
   if (!ws.vg_active) return;                               \
   const int n = ws.view_prefix[ws.nframes];                \
@@ -65,7 +65,7 @@ __global__ void __launch_bounds__(256) k_vg_bbox(DevBuffers d, int lane0) {
 __global__ void k_vg_plan(DevBuffers d, int lane0, int nlanes) {
   const int l = blockIdx.x * blockDim.x + threadIdx.x;
   if (l >= nlanes) return;
-  WinState& ws = d.wstate[lane0 + l];
+  WinState& ws = d.wstate[lane_at(d, lane0 + l)];
   if (!ws.vg_active) return;
   if (ws.vg_lo[0] == 0xffffffffu) {   // no finite point: the filtered cloud is empty
     ws.vg_passes = 0; ws.vg_div[0] = ws.vg_div[1] = ws.vg_div[2] = 0; ws.vg_invalid = 0u;
@@ -132,7 +132,7 @@ __global__ void __launch_bounds__(256) k_vg_hist(DevBuffers d, int lane0, int pa
 
 // exclusive scan of the lane's digit-major histogram (256 * tiles entries) by one CTA
 __global__ void __launch_bounds__(1024) k_vg_scan(DevBuffers d, int lane0, int pass) {
-  const int lane_b = lane0 + blockIdx.x;
+  const int lane_b = lane_at(d, lane0 + blockIdx.x);
   const WinState& ws = d.wstate[lane_b];
   if (!ws.vg_active || pass >= ws.vg_passes) return;
   const int n = ws.view_prefix[ws.nframes];
