@@ -36,7 +36,8 @@
 namespace {
 
 constexpr int kTile = 2048;            // keys per radix-sort block (256 threads x 8)
-constexpr int kMaxLatBits = 10;        // upper bound of the lattice bits per axis inside a coarse cell (MapDev::lat_bits)
+constexpr int kMaxCellVoxels = 1016;   // voxels per axis of one key's points: keeps PCL's per-cell int32 index space (1017^3) from overflowing
+constexpr int kRankBits = 16;          // touched-cell rank bits of the sort key (cap_cells = 2^16)
 constexpr unsigned long long kEmptyKey = ~0ull;
 
 struct MapState {      // device-resident scalars
@@ -52,8 +53,10 @@ struct MapState {      // device-resident scalars
 
 struct MapDev {
   double xy, inv_xy, xy_half, zs, inv_z, z_half;
+  double xy_slack, z_slack;  // 1 when size / 2 is not an integer (the key's int truncation then moves it up to 1 m), else 0
   float inv_leaf;
-  int lat_bits;          // bits per lattice axis of the sort key: ceil(log2(cell size / resolution + 8)); fewer bits = fewer radix passes
+  int lat_margin;        // lattice voxels kept below a key's lowest face for float rounding (grows with 1 / resolution)
+  int lat_bits;          // bits per lattice axis of the sort key, from the span one key covers; fewer bits = fewer radix passes
   int cap_points, cap_cells, hcap, cap_new;
   float4* pool[2];
   int* cell_count;       // [cap_cells] points per cell (creation order)
@@ -109,6 +112,16 @@ __device__ __forceinline__ int find_slot(const MapDev& m, unsigned long long key
 }
 
 __device__ __forceinline__ int lattice(float v, float inv_leaf) { return (int)floorf(v * inv_leaf); }
+
+// Lattice origin of a key along one axis: the lowest cell face the key can stand for, minus the margin.
+// The key int(floor(v / size) * size + size / 2) truncates toward zero, so when size / 2 is not an
+// integer a positive key lies up to 1 m below its cell's centre and a non-positive one up to 1 m above
+// it; below 2 m the cells -1 and 0 both give key 0, which then covers [-size, size).  The face is taken
+// in double: rounding it to float would move it by up to 0.06 m at the edge of the key range.
+__device__ __forceinline__ int lattice_origin(int key, double half, double slack, const MapDev& m) {
+  const double face = (double)key - half - (key <= 0 ? slack : 0.0);
+  return (int)floor(__dmul_rn(face, (double)m.inv_leaf)) - m.lat_margin;
+}
 
 // ---------------------------------------------------------------------------------------------------
 // Map::updateMap as ONE cooperative launch.  An update touches a few tens of thousands of points, so
@@ -318,11 +331,10 @@ __global__ void __launch_bounds__(kMapThreads) k_map_update(MapDev m, const floa
       if (cid < 0) { m.keys[0][wi] = kEmptyKey; m.vals[0][wi] = (unsigned)wi; continue; }  // dropped point: sorts last
       r = m.rank[cid];
     }
-    // lattice relative to the cell's lower corner (with a 2-voxel margin for float rounding at the faces)
-    const float fx = (float)((double)m.cell_key[cid * 3 + 0] - m.xy_half), fy = (float)((double)m.cell_key[cid * 3 + 1] - m.xy_half);
-    const float fz = (float)((double)m.cell_key[cid * 3 + 2] - m.z_half);
-    const int lx = lattice(p.x, m.inv_leaf) - (lattice(fx, m.inv_leaf) - 2), ly = lattice(p.y, m.inv_leaf) - (lattice(fy, m.inv_leaf) - 2);
-    const int lz = lattice(p.z, m.inv_leaf) - (lattice(fz, m.inv_leaf) - 2);
+    // lattice relative to the lowest face the cell's key can stand for
+    const int lx = lattice(p.x, m.inv_leaf) - lattice_origin(m.cell_key[cid * 3 + 0], m.xy_half, m.xy_slack, m);
+    const int ly = lattice(p.y, m.inv_leaf) - lattice_origin(m.cell_key[cid * 3 + 1], m.xy_half, m.xy_slack, m);
+    const int lz = lattice(p.z, m.inv_leaf) - lattice_origin(m.cell_key[cid * 3 + 2], m.z_half, m.z_slack, m);
     const int lim = 1 << m.lat_bits;
     if (lx < 0 || lx >= lim || ly < 0 || ly >= lim || lz < 0 || lz >= lim) atomicOr(&st.error, 4);
     m.keys[0][wi] = ((unsigned long long)r << (3 * m.lat_bits)) | ((unsigned long long)(lz & (lim - 1)) << (2 * m.lat_bits)) |
@@ -571,8 +583,23 @@ int liodom_map_create(double voxel_xysize, double voxel_zsize, double resolution
     return mfail(nullptr, LIODOM_E_INVALID, "bad arguments");
   if (voxel_xysize < 1.0 || voxel_zsize < 1.0)   // the reference's `int += double` cell loops (src/map.cc:157-186) never advance below 1 m
     return mfail(nullptr, LIODOM_E_INVALID, "voxel sizes below 1 m are not supported (the reference's getLocalMap loops do not terminate)");
-  const double vox = std::max(voxel_xysize, voxel_zsize) / resolution;
-  if (vox > (1 << kMaxLatBits) - 8) return mfail(nullptr, LIODOM_E_INVALID, "cell size / resolution = %.0f exceeds %d voxels per axis", vox, (1 << kMaxLatBits) - 8);
+  // Extent of one key's points per axis: its cell, or the two cells sharing key 0 below 2 m (lattice_origin).
+  auto extent = [](double s) { return s < 2.0 ? 2.0 * s : s; };
+  auto slack = [](double s) { return s / 2.0 == std::floor(s / 2.0) ? 0.0 : 1.0; };
+  const double vox = std::max(extent(voxel_xysize), extent(voxel_zsize)) / resolution;
+  if (vox > kMaxCellVoxels)
+    return mfail(nullptr, LIODOM_E_INVALID, "cell extent / resolution = %.0f exceeds %d voxels per axis (cells below 2 m count twice: key 0 holds two)",
+                 vox, kMaxCellVoxels);
+  // A point's float lattice index is off its exact value by at most half an ulp, <= |p| / res * 2^-24 <= 2^20 / res * 2^-24
+  // inside the key range; the origin keeps that much + 2 voxels below the lowest face, and the span as much above the top.
+  const float inv_leaf = 1.0f / (float)resolution;   // pcl::VoxelGrid: inverse_leaf_size_ in float
+  const int margin = 2 + (int)(inv_leaf / 16.0f);
+  const double span_m = std::max(extent(voxel_xysize) + slack(voxel_xysize), extent(voxel_zsize) + slack(voxel_zsize));
+  const long long span = (long long)std::ceil(span_m * inv_leaf) + 2 * margin + 2;
+  int lat_bits = 1;
+  while ((1ll << lat_bits) < span) ++lat_bits;
+  if (3 * lat_bits + kRankBits > 63)   // kEmptyKey must stay above every sort key
+    return mfail(nullptr, LIODOM_E_INVALID, "voxel lattice of %d bits per axis does not fit the 64-bit sort key", lat_bits);
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || device < 0 || device >= ndev)
     return mfail(nullptr, LIODOM_E_NODEVICE, "no usable CUDA device (count=%d, requested %d): liodom_b200 has no CPU fallback", ndev, device);
@@ -592,9 +619,10 @@ int liodom_map_create(double voxel_xysize, double voxel_zsize, double resolution
   MapDev& m = c->m;
   m.xy = voxel_xysize; m.inv_xy = 1.0 / voxel_xysize; m.xy_half = voxel_xysize / 2.0;   // src/map.cc:70-81
   m.zs = voxel_zsize; m.inv_z = 1.0 / voxel_zsize; m.z_half = voxel_zsize / 2.0;
-  m.inv_leaf = 1.0f / (float)resolution;   // pcl::VoxelGrid: inverse_leaf_size_ in float
-  m.lat_bits = 1;
-  while ((1 << m.lat_bits) < (int)std::ceil(vox) + 8) ++m.lat_bits;   // lattice span of a cell + the 2-voxel margins and rounding slack
+  m.xy_slack = slack(voxel_xysize); m.z_slack = slack(voxel_zsize);
+  m.inv_leaf = inv_leaf;
+  m.lat_margin = margin;
+  m.lat_bits = lat_bits;
   m.cap_points = max_points;
   m.cap_new = 1 << 16;
   m.cap_cells = 1 << 16;

@@ -161,12 +161,17 @@ def huber_cost(cab, q, t, a=0.2, min_range=3.0, max_range=75.0):
 
 def voxelgrid(pts, leaf):
     """pcl::VoxelGrid<PointXYZI> centroids per voxel, output in ascending voxel index
-    (App. A.3); in-voxel accumulation in input order (float32)."""
+    (App. A.3); in-voxel accumulation in input order (float32).  Non-finite points are skipped; when
+    PCL's (max - min) * inv + 1 product exceeds INT32_MAX the input is returned unchanged."""
     p = np.asarray(pts, np.float32)
+    p = p[np.isfinite(p[:, :3]).all(1)] if len(p) else p
     if len(p) == 0:
         return p.copy()
     inv = np.float32(1.0) / np.float32(leaf)
     mn, mx = p[:, :3].min(0), p[:, :3].max(0)
+    dd = [int(np.float32((mx[a] - mn[a]) * inv)) + 1 for a in range(3)]
+    if dd[0] * dd[1] * dd[2] > 2147483647:
+        return np.asarray(pts, np.float32).copy()
     minb = np.floor(mn * inv).astype(np.int64)
     maxb = np.floor(mx * inv).astype(np.int64)
     div = maxb - minb + 1
@@ -187,3 +192,31 @@ def map_cell_key(p, xy=40.0, z=50.0):
     inv_xy, inv_z = 1.0 / xy, 1.0 / z
     return (int(np.floor(p[0] * inv_xy) * xy + xy / 2.0), int(np.floor(p[1] * inv_xy) * xy + xy / 2.0),
             int(np.floor(p[2] * inv_z) * z + z / 2.0))
+
+
+class Map:
+    """Map::updateMap / getMap (src/map.cc:90-139): a dict keyed by the int key triple in creation order;
+    every touched cell is re-filtered by `voxelgrid` over its old centroids followed by its new points."""
+
+    def __init__(self, xy, z, resolution):
+        self.xy, self.z, self.leaf = xy, z, np.float32(resolution)
+        self.cells = {}
+
+    def update(self, pts, T):
+        p = transform(pts, T)
+        touched = {}
+        for row in p:
+            k = map_cell_key(row.astype(np.float64), self.xy, self.z)
+            self.cells.setdefault(k, np.zeros((0, 4), np.float32))
+            touched.setdefault(k, []).append(row)
+        for k, rows in touched.items():
+            self.cells[k] = voxelgrid(np.concatenate([self.cells[k], np.array(rows, np.float32)]), self.leaf)
+
+    def keys(self):
+        return np.array(list(self.cells), np.int32).reshape(-1, 3)
+
+    def counts(self):
+        return np.array([len(v) for v in self.cells.values()], np.int32)
+
+    def get_map(self):
+        return np.concatenate(list(self.cells.values())) if self.cells else np.zeros((0, 4), np.float32)
