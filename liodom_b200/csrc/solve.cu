@@ -107,16 +107,17 @@ __device__ void lm_after_jacobian(LmCtrl& c, const double* acc) {
   for (int k = 0; k < 21; ++k) c.H[k] = acc[k];
   for (int k = 0; k < 6; ++k) c.g[k] = acc[21 + k];
   c.x_cost = acc[27];
-  c.sum.jac_evals++;
   if (c.first) {
     c.sum.num_residual_blocks = (int)(acc[28] + 0.5);
     c.sum.initial_cost = c.x_cost;
+    c.first = 0;
+    if (c.sum.num_residual_blocks == 0) return lm_done(c, 4);   // nothing to solve: no evaluation is counted
     for (int j = 0; j < 6; ++j) c.scale[j] = 1.0 / (1.0 + sqrt(c.H[hidx(j, j)]));  // jacobi_scaling, once
     double s = 0.0; for (int k = 0; k < 7; ++k) s += c.x[k] * c.x[k];
     c.x_norm = sqrt(s);
-    c.step_is_successful = 1; c.iteration = 0; c.first = 0;
-    if (c.sum.num_residual_blocks == 0) return lm_done(c, 4);
+    c.step_is_successful = 1; c.iteration = 0;
   }
+  c.sum.jac_evals++;
   double ng[6], xp[7];
   for (int j = 0; j < 6; ++j) ng[j] = -c.g[j];
   state_plus(c.x, ng, xp);

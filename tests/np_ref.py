@@ -159,6 +159,187 @@ def huber_cost(cab, q, t, a=0.2, min_range=3.0, max_range=75.0):
     return cost
 
 
+def _blocks_eval(cab, x, min_range, max_range, jac):
+    """All residual blocks at x = (qx, qy, qz, qw, tx, ty, tz), vectorised: Huber-corrected residuals [3n], Jacobian
+    [3n, 6] in the tangent space (A.4, A.5) and the cost.  The rows of a block are scaled by sqrt(rho') (the Corrector
+    with rho'' <= 0).  q is used as given, unit or not."""
+    cab = np.asarray(cab, float).reshape(-1, 9)
+    c, a, b = cab[:, 0:3], cab[:, 3:6], cab[:, 6:9]
+    qv, qw, t = np.asarray(x[:3], float), float(x[3]), np.asarray(x[4:7], float)
+    uv = 2.0 * np.cross(qv, c)
+    u = c + qw * uv + np.cross(qv, uv)               # Eigen q * c
+    lp = u + t
+    nu = np.cross(lp - a, lp - b)
+    de = a - b
+    with np.errstate(divide="ignore", invalid="ignore"):
+        inv_den = 1.0 / np.sqrt(np.sum(de * de, 1))
+        pxy = c[:, :2] - t[:2]
+        rho = np.sqrt(np.sum(pxy * pxy, 1))
+        w = 1.01 - (rho - min_range) / (max_range - min_range)
+        r = (w * inv_den)[:, None] * nu
+        s = np.sum(r * r, 1)
+        big = s > 0.04                                   # HuberLoss(0.2); NaN takes the quadratic branch, as in Ceres
+        sq = np.sqrt(np.where(big, s, 0.0))
+        rho0 = np.where(big, 0.4 * sq - 0.04, s)
+        rho1 = np.where(big, np.maximum(np.finfo(float).tiny, 0.2 / np.where(big, sq, 1.0)), 1.0)
+        sc = np.sqrt(rho1)
+        cost = 0.5 * float(np.sum(rho0))
+        rs = (sc[:, None] * r).reshape(-1)
+        if not jac:
+            return rs, None, cost
+        # d lp / d delta: q+ = dq (x) q with |dq| = 1, and Eigen's q * c equals the sandwich q c q* + (1 - |q|^2) c, so
+        # the tangent derivative is 2 e_k x S with S = q c q* = u - (1 - |q|^2) c (for unit q, S = u = R c).
+        S = u - (1.0 - float(qv @ qv + qw * qw)) * c
+        n = len(cab)
+        J = np.empty((n, 3, 6))
+        wd = (w * inv_den * sc)[:, None]
+        for k in range(3):
+            e = np.zeros(3)
+            e[k] = 1.0
+            dlp = 2.0 * np.cross(e, S)
+            J[:, :, k] = wd * np.cross(-de, dlp)                        # d nu / d lp = [b - a]x
+            J[:, :, 3 + k] = wd * np.cross(-de, np.broadcast_to(e, de.shape))
+        dw = np.zeros((n, 3))
+        dw[:, :2] = pxy / (rho[:, None] * (max_range - min_range))     # d w / d t
+        nd = (inv_den * sc)[:, None] * nu
+        J[:, :, 3:] += nd[:, :, None] * dw[:, None, :]
+    return rs, J.reshape(-1, 6), cost
+
+
+def _state_plus(x, d6):
+    return np.concatenate([quat_plus(x[:4], d6[:3]), np.asarray(x[4:7], float) + d6[3:]])
+
+
+def lm_solve(cab, q, t, min_range=3.0, max_range=75.0, max_iterations=4):
+    """ceres::Solve as the reference configures it (SURVEY.md App. A.5): trust-region Levenberg-Marquardt, Jacobi
+    scaling computed once, LM diagonal clamped to [1e-6, 1e32], the augmented system [J_s; D] solved by Householder QR,
+    model cost change from J, the rho test, the radius update and the three tolerances.
+
+    -> (q, t, summary); summary has the fields of oracle.SolveSummary plus `rejected_steps`, `invalid_steps` and
+    `cond_first` = cond(J_s'J_s + D^2) of the first trust-region step (NaN when none was computed)."""
+    from types import SimpleNamespace
+    cab = np.asarray(cab, float).reshape(-1, 9)
+    n = len(cab)
+    S = SimpleNamespace(iterations=0, successful_steps=0, termination=0, initial_cost=0.0, final_cost=0.0,
+                        num_residual_blocks=n, cost_evals=0, jac_evals=0, rejected_steps=0, invalid_steps=0,
+                        cond_first=float("nan"))
+    x = np.concatenate([np.asarray(q, float), np.asarray(t, float)])
+    if n == 0:
+        S.termination = 4
+        return x[:4].copy(), x[4:].copy(), S
+
+    def grad_max_norm(x, g):
+        # ||x - Plus(x, -g)||_inf; a NaN component is dropped (std::max / fmax keep the other operand)
+        d = np.abs(_state_plus(x, -g) - x)
+        d = d[~np.isnan(d)]
+        return float(d.max(initial=0.0))
+
+    r, J, cost = _blocks_eval(cab, x, min_range, max_range, True)
+    S.jac_evals += 1
+    S.initial_cost = cost
+    scale = 1.0 / (1.0 + np.sqrt(np.sum(J * J, 0)))
+    g = J.T @ r
+    gmax = grad_max_norm(x, g)
+    radius, decrease = 1e4, 2.0
+    reuse, success, invalid = False, True, 0
+    diagonal = None
+    while True:
+        if S.iterations >= max_iterations:
+            S.termination = 0
+            break
+        if success and gmax <= 1e-10:
+            S.termination = 1
+            break
+        if radius < 1e-32:
+            S.termination = 5
+            break
+        S.iterations += 1
+        Js = J * scale
+        if not reuse:
+            diagonal = np.minimum(np.maximum(np.sum(Js * Js, 0), 1e-6), 1e32)
+        D = np.sqrt(diagonal / radius)
+        if np.isnan(S.cond_first):
+            S.cond_first = float(np.linalg.cond(Js.T @ Js + np.diag(D * D)))
+        reuse = True
+        A = np.vstack([Js, np.diag(D)])
+        rhs = np.concatenate([r, np.zeros(6)])
+        mcc = -np.inf
+        if np.isfinite(A).all() and np.isfinite(rhs).all():
+            Q, R = np.linalg.qr(A)
+            y = np.linalg.solve(R, Q.T @ rhs)
+            if np.isfinite(y).all():
+                step = -y
+                m = Js @ step
+                mcc = -float(m @ (r + m / 2.0))
+        if not mcc > 0.0:                                   # invalid step
+            S.invalid_steps += 1
+            invalid += 1
+            if invalid >= 5:
+                S.termination = 5
+                break
+            radius *= 0.5
+            success = False
+            continue
+        invalid = 0
+        xc = _state_plus(x, step * scale)
+        _, _, cc = _blocks_eval(cab, xc, min_range, max_range, False)
+        S.cost_evals += 1
+        if not np.isfinite(cc):
+            cc = cost
+        if np.linalg.norm(x - xc) <= 1e-8 * (np.linalg.norm(x) + 1e-8):
+            S.termination = 2
+            break
+        change = cost - cc
+        if abs(change) <= 1e-6 * cost:
+            S.termination = 3
+            break
+        rel = change / mcc
+        if rel > 1e-3:                                      # accept
+            x = xc
+            r, J, cost = _blocks_eval(cab, x, min_range, max_range, True)
+            S.jac_evals += 1
+            g = J.T @ r
+            gmax = grad_max_norm(x, g)
+            S.successful_steps += 1
+            radius = min(1e16, radius / max(1.0 / 3.0, 1.0 - (2.0 * rel - 1.0) ** 3))
+            decrease, reuse, success = 2.0, False, True
+        else:                                               # reject
+            S.rejected_steps += 1
+            success = False
+            radius /= decrease
+            decrease *= 2.0
+    S.final_cost = cost
+    return x[:4].copy(), x[4:].copy(), S
+
+
+def exact_cost(cab, q, t, min_range=3.0, max_range=75.0):
+    """The Huber cost at one point, every block in 40-digit arithmetic from the double inputs (mpmath)."""
+    import mpmath
+    old = mpmath.mp.dps
+    mpmath.mp.dps = 40
+    try:
+        F = mpmath.mpf
+        qx, qy, qz, qw = (F(float(v)) for v in q)
+        tx, ty, tz = (F(float(v)) for v in t)
+        lo, span = F(float(min_range)), F(float(max_range)) - F(float(min_range))
+        total = F(0)
+        for row in np.asarray(cab, float).reshape(-1, 9):
+            cx, cy, cz, ax, ay, az, bx, by, bz = (F(float(v)) for v in row)
+            ux, uy, uz = 2 * (qy * cz - qz * cy), 2 * (qz * cx - qx * cz), 2 * (qx * cy - qy * cx)
+            lx = cx + qw * ux + (qy * uz - qz * uy) + tx
+            ly = cy + qw * uy + (qz * ux - qx * uz) + ty
+            lz = cz + qw * uz + (qx * uy - qy * ux) + tz
+            pax, pay, paz, pbx, pby, pbz = lx - ax, ly - ay, lz - az, lx - bx, ly - by, lz - bz
+            nx, ny, nz = pay * pbz - paz * pby, paz * pbx - pax * pbz, pax * pby - pay * pbx
+            den2 = (ax - bx) ** 2 + (ay - by) ** 2 + (az - bz) ** 2
+            w = F(1.01) - (mpmath.sqrt((cx - tx) ** 2 + (cy - ty) ** 2) - lo) / span
+            s = w * w * (nx * nx + ny * ny + nz * nz) / den2
+            total += s / 2 if s <= F(0.04) else (F(0.4) * mpmath.sqrt(s) - F(0.04)) / 2   # the double constants
+        return total
+    finally:
+        mpmath.mp.dps = old
+
+
 def voxelgrid(pts, leaf):
     """pcl::VoxelGrid<PointXYZI> centroids per voxel, output in ascending voxel index
     (App. A.3); in-voxel accumulation in input order (float32).  Non-finite points are skipped; when

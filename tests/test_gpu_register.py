@@ -214,6 +214,14 @@ def _run_teacher_forced(sensor, seed, nframes, okw, gkw, max_points, traj=0, wid
             for it in range(2):
                 assert gd.n_map[it] == od.n_map[it]
                 assert gd.n_matches[it] == od.n_matches[it] or it == 1, (f, it, gd.n_matches[it], od.n_matches[it])
+                if gd.n_matches[it] != od.n_matches[it]:
+                    continue   # outer iteration 1 may see other matches when the first solves differ in the last bits
+                g, o = gd.solve[it], od.solve[it]
+                gi = (g.iterations, g.successful_steps, g.termination, g.num_residual_blocks, g.cost_evals, g.jac_evals)
+                oi = (o.iterations, o.successful_steps, o.termination, o.num_residual_blocks, o.cost_evals, o.jac_evals)
+                assert gi == oi and g.num_residual_blocks == gd.n_matches[it], (f, it, gi, oi)
+                assert abs(g.initial_cost - o.initial_cost) <= 1e-9 * max(1.0, o.initial_cost), (f, it)
+                assert abs(g.final_cost - o.final_cost) <= 1e-7 * max(1.0, o.final_cost), (f, it)
         dt, dr = pose_err(gpose, opose)
         assert dt < TOL_T and dr < TOL_R, "frame %d: %g m, %g rad" % (f, dt, dr)
         worst = (max(worst[0], dt), max(worst[1], dr))
