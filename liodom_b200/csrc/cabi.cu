@@ -15,10 +15,6 @@
 
 using namespace liodom;
 
-namespace liodom {
-int launch_hash_begin_only(const DevBuffers& d, cudaStream_t s, int lane);
-}
-
 struct liodom_ctx {
   liodom_params params;
   int device = 0;
@@ -63,14 +59,10 @@ struct liodom_ctx {
   // optional per-stage device timing of liodom_scan_batch (bench roofline evidence)
   bool stage_timing = false;
   std::vector<cudaEvent_t> stage_events;  // LIODOM_NUM_STAGES + 1 events per timed call
-  // LIODOM_TIMELINE=1: copy start/end and compute start/end of every liodom_scan_batch, printed at destroy
-  bool timeline = false;
-  std::vector<cudaEvent_t> tl_events;
 };
 
-// Record a stage boundary on the compute stream when stage timing is on.
+// Record a stage boundary on the compute stream (stage timing).
 static void stage_mark(liodom_ctx* c) {
-  if (!c->stage_timing) return;
   cudaEvent_t e = nullptr;
   if (cudaEventCreate(&e) != cudaSuccess) return;
   cudaEventRecord(e, c->stream);
@@ -137,6 +129,14 @@ static int hash_generation_guard(liodom_ctx* c, unsigned upcoming_builds) {
   return 0;
 }
 
+// Odometry state of a lane that has seen no scan: identity poses, rotations and laser-to-base transform.
+static OdomState identity_odom_state() {
+  OdomState os; std::memset(&os, 0, sizeof(os));
+  os.odom[0] = os.odom[5] = os.odom[10] = 1.0; os.prev[0] = os.prev[5] = os.prev[10] = 1.0; os.q[3] = 1.0;
+  os.imu_q[3] = 1.0; os.l2b[0] = os.l2b[5] = os.l2b[10] = 1.0;
+  return os;
+}
+
 extern "C" {
 
 void liodom_default_params(liodom_params* p) {
@@ -189,7 +189,6 @@ int liodom_ctx_create(const liodom_params* up, int batch, int device, liodom_ctx
   CKC(cudaSetDevice(device));
   CKC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   CKC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-  c->timeline = getenv("LIODOM_TIMELINE") != nullptr;
   {
     int g = default_lane_groups(batch);
     if (const char* e = getenv("LIODOM_LANE_GROUPS")) { g = atoi(e); c->groups_forced = true; }
@@ -307,17 +306,9 @@ int liodom_ctx_create(const liodom_params* up, int batch, int device, liodom_ctx
   c->dprod.gate = nullptr; c->dprod.knn_idx = nullptr; c->dprod.knn_d2 = nullptr; c->dprod.eig = nullptr;
   c->dprod.q_world = nullptr; c->dprod.src_index = nullptr;
   // initial state: identity poses, empty windows
-  std::vector<OdomState> os(B);
+  std::vector<OdomState> os(B, identity_odom_state());
   std::vector<WinState> ws(B);
-  for (size_t l = 0; l < B; ++l) {
-    std::memset(&os[l], 0, sizeof(OdomState)); std::memset(&ws[l], 0, sizeof(WinState));
-    os[l].odom[0] = os[l].odom[5] = os[l].odom[10] = 1.0;
-    os[l].prev[0] = os[l].prev[5] = os[l].prev[10] = 1.0;
-    os[l].q[3] = 1.0;
-    os[l].imu_q[3] = 1.0;
-    os[l].l2b[0] = os[l].l2b[5] = os[l].l2b[10] = 1.0;
-    ws[l].max_frames = P.prev_frames;
-  }
+  for (size_t l = 0; l < B; ++l) { std::memset(&ws[l], 0, sizeof(WinState)); ws[l].max_frames = P.prev_frames; }
   CKC(cudaMemcpyAsync(d.ostate, os.data(), sizeof(OdomState) * B, cudaMemcpyHostToDevice, c->stream));
   CKC(cudaMemcpyAsync(d.wstate, ws.data(), sizeof(WinState) * B, cudaMemcpyHostToDevice, c->stream));
   CKC(cudaStreamSynchronize(c->stream));
@@ -331,14 +322,6 @@ void liodom_ctx_destroy(liodom_ctx* c) {
   cudaSetDevice(c->device);
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-  if (c->timeline && c->tl_events.size() >= 4) {
-    for (size_t k = 0; k + 3 < c->tl_events.size(); k += 4) {
-      float t[4];
-      for (int j = 0; j < 4; ++j) cudaEventElapsedTime(&t[j], c->tl_events[0], c->tl_events[k + j]);
-      fprintf(stderr, "[liodom timeline] step %zu: copy %.3f..%.3f  compute %.3f..%.3f ms\n", k / 4, t[0], t[1], t[2], t[3]);
-    }
-    for (cudaEvent_t e : c->tl_events) cudaEventDestroy(e);
-  }
   for (void* p : c->allocs) cudaFree(p);
   for (int k = 0; k < 2; ++k) {
     if (c->dev_in[k]) cudaFree(c->dev_in[k]);
@@ -452,6 +435,88 @@ static void copy_summary(const SolveSummaryDev& s, liodom_solve_summary* o) {
   o->initial_cost = s.initial_cost; o->final_cost = s.final_cost;
 }
 
+static void copy_diag(const FrameDiagDev& g, liodom_frame_diag* o) {
+  o->n_edges = g.n_edges;
+  for (int k = 0; k < 2; ++k) { o->n_map[k] = g.n_map[k]; o->n_matches[k] = g.n_matches[k]; copy_summary(g.solve[k], &o->solve[k]); }
+  std::memcpy(o->pred_pose, g.pred_pose, sizeof(g.pred_pose));
+}
+
+// ---- step orchestration ------------------------------------------------------------------
+// The stages of a scan step, in the order of api.STAGE_NAMES (liodom_stage_times reports one time per stage).
+enum Stage { kSplit, kExtract, kAssoc0, kSolve0, kAssoc1, kSolve1, kWindow, kNumStages };
+static_assert(kNumStages == LIODOM_NUM_STAGES, "one stage time per Stage");
+
+// The kernels of one stage for the positions lr on stream s; returns how many it launched.  sc (a point-sharded
+// scan, else null): extraction of this rank's rings and an all-gather of the edge slots, association and solve of
+// this rank's share of the edges.  NCCL return codes go to *nccl_rc.
+static int enqueue_stage(const DevBuffers& d, cudaStream_t s, LaneRange lr, Stage st, bool want_keys, const ShardComm* sc,
+                         int* nccl_rc) {
+  int k = 0;
+  switch (st) {
+    case kSplit: return launch_split(d, s, lr);
+    case kExtract:
+      if (!sc) {
+        k += launch_extract_rings(d, s, lr, 0, d.p.scan_lines, want_keys);
+      } else {
+        const int per = d.p.scan_lines / sc->world;
+        const size_t slots_per_rank = (size_t)per * d.p.scan_regions * (d.p.edges_per_region + 1);
+        k += launch_extract_rings(d, s, lr, sc->rank * per, per, want_keys);
+        *nccl_rc |= shard_group_start();
+        *nccl_rc |= shard_allgather_bytes(sc, d.slots, slots_per_rank * sizeof(float4), s);
+        *nccl_rc |= shard_allgather_bytes(sc, d.slot_idx, slots_per_rank * sizeof(int), s);
+        *nccl_rc |= shard_allgather_bytes(sc, d.region_cnt, (size_t)per * d.p.scan_regions * sizeof(int), s);
+        *nccl_rc |= shard_group_end();
+      }
+      return k + launch_compact(d, s, lr);
+    case kAssoc0:
+    case kAssoc1: {
+      const int it = st == kAssoc1;   // src/laser_odometry.cc:198
+      if (it == 0) k += launch_predict(d, s, lr);
+      return k + (sc ? launch_associate_shard(d, s, lr.lane0, it, sc->rank, sc->world)
+                     : launch_associate(d, s, lr, it, false, nullptr));
+    }
+    case kSolve0:
+    case kSolve1: {
+      const int it = st == kSolve1;
+      return sc ? launch_solve_shard(d, s, lr.lane0, it, sc, nccl_rc) : launch_solve(d, s, lr, it);
+    }
+    default: return launch_window_update(d, s, lr);
+  }
+}
+
+// Stages [first, last) for the positions lr.  G == 1: on the compute stream, with an event before the first stage and
+// after each one when `timed`.  G > 1: the positions are cut into G groups whose chains run on their own streams,
+// enqueued stage by stage across the groups, so that the tail of one group's latency-bound kernels (k_associate,
+// k_solve) overlaps another group's work.
+static int enqueue_stages(liodom_ctx* c, const DevBuffers& d, LaneRange lr, Stage first, Stage last, int G, bool timed,
+                          bool want_keys, const ShardComm* sc) {
+  int k = 0, nrc = 0;
+  if (G == 1) {
+    if (timed) stage_mark(c);
+    for (int st = first; st < last; ++st) {
+      k += enqueue_stage(d, c->stream, lr, (Stage)st, want_keys, sc, &nrc);
+      if (timed) stage_mark(c);
+    }
+  } else {
+    // fork: every group's chain waits for the descriptors (and the H2D copy) on the main stream
+    CK(cudaEventRecord(c->ev_fork, c->stream));
+    for (int g = 0; g < G; ++g) CK(cudaStreamWaitEvent(c->group_stream[g], c->ev_fork, 0));
+    for (int st = first; st < last; ++st)
+      for (int g = 0; g < G; ++g) {
+        const int l0 = (int)((long long)lr.nlanes * g / G), l1 = (int)((long long)lr.nlanes * (g + 1) / G);
+        k += enqueue_stage(d, c->group_stream[g], LaneRange{lr.lane0 + l0, l1 - l0}, (Stage)st, want_keys, sc, &nrc);
+      }
+    for (int g = 0; g < G; ++g) {   // join
+      CK(cudaEventRecord(c->ev_join[g], c->group_stream[g]));
+      CK(cudaStreamWaitEvent(c->stream, c->ev_join[g], 0));
+    }
+  }
+  if (nrc != 0) return fail(c, LIODOM_E_CUDA, "NCCL call failed in the point-sharded scan: %s", shard_error_string(nrc));
+  c->launches += k;
+  CK(cudaGetLastError());
+  return 0;
+}
+
 extern "C" {
 
 int liodom_split(liodom_ctx* c, int lane, const void* pts, int n, int stride_bytes, int width, int height,
@@ -462,8 +527,7 @@ int liodom_split(liodom_ctx* c, int lane, const void* pts, int n, int stride_byt
   rc = layout_from_stride(c, stride_bytes, &lay); if (rc) return rc;
   rc = stage_scan(c, lane, pts, n, lay, width, height); if (rc) return rc;
   const DevBuffers& d = c->d;
-  c->launches += launch_split(d, c->stream, LaneRange{lane, 1});
-  CK(cudaGetLastError());
+  rc = enqueue_stages(c, d, LaneRange{lane, 1}, kSplit, kExtract, 1, false, false, nullptr); if (rc) return rc;
   const int L = d.p.scan_lines;
   std::vector<int32_t> off(L + 1);
   std::vector<uint8_t> rid(n > 0 ? n : 1);
@@ -506,9 +570,7 @@ static int extract_impl(liodom_ctx* c, int lane, const void* pts, int n, const L
   int rc = stage_scan(c, lane, pts, n, lay, width, height); if (rc) return rc;
   const DevBuffers& d = c->dprod;
   if (keys) CK(cudaMemsetAsync(d.keys + (size_t)lane * d.p.Ncap, 0xff, sizeof(double) * d.p.Ncap, c->stream));  // NaN
-  c->launches += launch_split(d, c->stream, LaneRange{lane, 1});
-  c->launches += launch_extract(d, c->stream, LaneRange{lane, 1}, keys != nullptr);
-  CK(cudaGetLastError());
+  rc = enqueue_stages(c, d, LaneRange{lane, 1}, kSplit, kAssoc0, 1, false, keys != nullptr, nullptr); if (rc) return rc;
   OdomState os;
   CK(cudaMemcpyAsync(&os, d.ostate + lane, sizeof(os), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
@@ -611,9 +673,7 @@ int liodom_commit_received_map(liodom_ctx* c, int lane, int n) {
 
 int liodom_odom_reset(liodom_ctx* c, int lane) {
   int rc = check_lane(c, lane); if (rc) return rc;
-  OdomState os; std::memset(&os, 0, sizeof(os));
-  os.odom[0] = os.odom[5] = os.odom[10] = 1.0; os.prev[0] = os.prev[5] = os.prev[10] = 1.0; os.q[3] = 1.0;
-  os.imu_q[3] = 1.0; os.l2b[0] = os.l2b[5] = os.l2b[10] = 1.0;
+  const OdomState os = identity_odom_state();
   CK(cudaMemcpyAsync(c->d.ostate + lane, &os, sizeof(os), cudaMemcpyHostToDevice, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   return liodom_lmap_clear(c, lane);
@@ -700,54 +760,6 @@ int liodom_solve(liodom_ctx* c, int lane, const double* cab, int n, double* q4, 
   return 0;
 }
 
-static int enqueue_register(liodom_ctx* c, const DevBuffers& d, LaneRange lr) {
-  int k = 0;
-  k += launch_predict(d, c->stream, lr);
-  for (int it = 0; it < 2; ++it) {  // src/laser_odometry.cc:198
-    k += launch_associate(d, c->stream, lr, it, false, nullptr);
-    stage_mark(c);
-    k += launch_solve(d, c->stream, lr, it);
-    stage_mark(c);
-  }
-  k += launch_window_update(d, c->stream, lr);
-  stage_mark(c);
-  return k;
-}
-
-// Point-sharded scan (one lane): ring-sharded extraction + all-gather of the edge slots, replicated
-// prediction / ordering / window, edge-sharded association and solve with a 29-double all-reduce per
-// LM evaluation.
-static int enqueue_scan_sharded(liodom_ctx* c, const DevBuffers& d, int* launches) {
-  const ShardComm* sc = &c->shard;
-  const LaneRange lr{0, 1};
-  const int L = d.p.scan_lines, per = L / sc->world;
-  const size_t slots_per_rank = (size_t)per * d.p.scan_regions * (d.p.edges_per_region + 1);
-  int k = 0, nrc = 0;
-  stage_mark(c);
-  k += launch_split(d, c->stream, lr);
-  stage_mark(c);
-  k += launch_extract_rings(d, c->stream, lr, sc->rank * per, per);
-  nrc |= shard_group_start();
-  nrc |= shard_allgather_bytes(sc, d.slots, slots_per_rank * sizeof(float4), c->stream);
-  nrc |= shard_allgather_bytes(sc, d.slot_idx, slots_per_rank * sizeof(int), c->stream);
-  nrc |= shard_allgather_bytes(sc, d.region_cnt, (size_t)per * d.p.scan_regions * sizeof(int), c->stream);
-  nrc |= shard_group_end();
-  k += launch_compact(d, c->stream, lr);
-  stage_mark(c);
-  k += launch_predict(d, c->stream, lr);
-  for (int it = 0; it < 2; ++it) {
-    k += launch_associate_shard(d, c->stream, 0, it, sc->rank, sc->world);
-    stage_mark(c);
-    k += launch_solve_shard(d, c->stream, 0, it, sc, &nrc);
-    stage_mark(c);
-  }
-  k += launch_window_update(d, c->stream, lr);
-  stage_mark(c);
-  *launches = k;
-  if (nrc != 0) return fail(c, LIODOM_E_CUDA, "NCCL call failed in the point-sharded scan: %s", shard_error_string(nrc));
-  return 0;
-}
-
 int liodom_shard_unique_id(char id_out[128]) {
   const int rc = shard_unique_id(id_out);
   if (rc != 0) return fail(nullptr, LIODOM_E_INVALID, "ncclGetUniqueId: %s", shard_error_string(rc));
@@ -772,20 +784,15 @@ int liodom_register(liodom_ctx* c, int lane, const float* edges_xyzi, int n_edge
   rc = hash_generation_guard(c, 1); if (rc) return rc;
   rc = put_edges(c, lane, edges_xyzi, n_edges); if (rc) return rc;
   const DevBuffers& d = c->dprod;
-  const bool st = c->stage_timing;  // stage timing covers liodom_scan_batch only
-  c->stage_timing = false;
-  c->launches += enqueue_register(c, d, LaneRange{lane, 1});
-  c->stage_timing = st;
-  CK(cudaGetLastError());
+  rc = enqueue_stages(c, d, LaneRange{lane, 1}, kAssoc0, kNumStages, 1, false, false, nullptr); if (rc) return rc;
   double pose[16]; FrameDiagDev dg;
   CK(cudaMemcpyAsync(pose, d.poses_out + (size_t)lane * 16, sizeof(pose), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaMemcpyAsync(&dg, d.diag + lane, sizeof(dg), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   if (pose16_out) std::memcpy(pose16_out, pose, sizeof(pose));
   if (diag) {
-    diag->n_edges = n_edges;
-    for (int k = 0; k < 2; ++k) { diag->n_map[k] = dg.n_map[k]; diag->n_matches[k] = dg.n_matches[k]; copy_summary(dg.solve[k], &diag->solve[k]); }
-    std::memcpy(diag->pred_pose, dg.pred_pose, sizeof(dg.pred_pose));
+    copy_diag(dg, diag);
+    diag->n_edges = n_edges;   // dg.n_edges is the count of the last extraction
   }
   return 0;
 }
@@ -880,7 +887,6 @@ static int scan_batch_impl(liodom_ctx* c, const int32_t* lanes, int n_lanes, con
     // queue behind the next scan's bulk copy on the same copy engine and stall this scan's kernels for
     // the whole transfer (measured: 6.6 ms instead of 2.7 ms of compute per second step at 128 lanes).
     CK(cudaMemcpyAsync(c->d_scan[buf], hd, desc_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-    if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->copy_stream); c->tl_events.push_back(e); }
     if (packed) {
       if (total > 0) CK(cudaMemcpyAsync(c->dev_in[buf], pts[0], total, cudaMemcpyHostToDevice, c->copy_stream));
     } else {
@@ -889,10 +895,8 @@ static int scan_batch_impl(liodom_ctx* c, const int32_t* lanes, int n_lanes, con
         if (bytes > 0) CK(cudaMemcpyAsync(const_cast<void*>(hd[lane_of(i)].pts), pts[i], bytes, cudaMemcpyHostToDevice, c->copy_stream));
       }
     }
-    if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->copy_stream); c->tl_events.push_back(e); }
     CK(cudaEventRecord(c->ev_copied[buf], c->copy_stream));
     CK(cudaStreamWaitEvent(c->stream, c->ev_copied[buf], 0));
-    if (c->timeline) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->stream); c->tl_events.push_back(e); }
   } else {
     for (int i = 0; i < n_lanes; ++i) fill_desc(&hd[lane_of(i)], pts[i], n[i], lay, width, height);
     CK(cudaMemcpyAsync(c->d_scan[buf], hd, desc_bytes, cudaMemcpyHostToDevice, c->stream));
@@ -900,52 +904,14 @@ static int scan_batch_impl(liodom_ctx* c, const int32_t* lanes, int n_lanes, con
   DevBuffers d = c->dprod;
   d.scan = c->d_scan[buf];
   d.lanes = lanes ? lane_list(c->d_scan[buf], B) : nullptr;
-  const LaneRange lr{0, n_lanes};
-  // the lane groups a context of n_lanes lanes would use, at most the streams this one has
-  const int G = std::min(std::min(c->groups, n_lanes), c->groups_forced ? c->groups : default_lane_groups(n_lanes));
-  int k = 0;
-  if (c->shard.world > 1) {
-    rc = enqueue_scan_sharded(c, d, &k);
-    if (rc) return rc;
-  } else if (G > 1 && !c->stage_timing) {
-    // fork: every group's chain waits for the descriptors (and the H2D copy) on the main stream
-    CK(cudaEventRecord(c->ev_fork, c->stream));
-    for (int g = 0; g < G; ++g) CK(cudaStreamWaitEvent(c->group_stream[g], c->ev_fork, 0));
-    for (int st = 0; st < 7; ++st)
-      for (int g = 0; g < G; ++g) {
-        const int l0 = (int)((long long)n_lanes * g / G), l1 = (int)((long long)n_lanes * (g + 1) / G);
-        const LaneRange gr{l0, l1 - l0};
-        cudaStream_t s = c->group_stream[g];
-        {
-          switch (st) {
-            case 0: k += launch_split(d, s, gr); break;
-            case 1: k += launch_extract(d, s, gr, false); break;
-            case 2: k += launch_predict(d, s, gr); k += launch_associate(d, s, gr, 0, false, nullptr); break;
-            case 3: k += launch_solve(d, s, gr, 0); break;
-            case 4: k += launch_associate(d, s, gr, 1, false, nullptr); break;
-            case 5: k += launch_solve(d, s, gr, 1); break;
-            default: k += launch_window_update(d, s, gr); break;
-          }
-        }
-      }
-    for (int g = 0; g < G; ++g) {   // join
-      CK(cudaEventRecord(c->ev_join[g], c->group_stream[g]));
-      CK(cudaStreamWaitEvent(c->stream, c->ev_join[g], 0));
-    }
-  } else {
-    stage_mark(c);
-    k += launch_split(d, c->stream, lr);
-    stage_mark(c);
-    k += launch_extract(d, c->stream, lr, false);
-    stage_mark(c);
-    k += enqueue_register(c, d, lr);
-  }
-  c->launches += k;
-  CK(cudaGetLastError());
+  // the lane groups a context of n_lanes lanes would use, at most the streams this one has; stage timing needs one
+  const int G = c->stage_timing ? 1 : std::min(std::min(c->groups, n_lanes), c->groups_forced ? c->groups : default_lane_groups(n_lanes));
+  rc = enqueue_stages(c, d, LaneRange{0, n_lanes}, kSplit, kNumStages, G, c->stage_timing, false,
+                      c->shard.world > 1 ? &c->shard : nullptr);
+  if (rc) return rc;
   CK(cudaMemcpyAsync(c->h_poses[buf], d.poses_out, sizeof(double) * 16 * B, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaMemcpy2DAsync(c->h_nedges[buf], sizeof(int), &d.ostate[0].n_edges, sizeof(OdomState), sizeof(int), B, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaEventRecord(c->ev_done[buf], c->stream));
-  if (c->timeline && !on_device) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, c->stream); c->tl_events.push_back(e); }
   c->in_flight[buf] = true;
   c->cur = buf;
   c->partial[buf] = n_lanes < B;
@@ -1008,9 +974,7 @@ int liodom_scan_diag(liodom_ctx* c, int lane, liodom_frame_diag* diag) {
   FrameDiagDev dg;
   CK(cudaMemcpyAsync(&dg, c->d.diag + lane, sizeof(dg), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
-  diag->n_edges = dg.n_edges;
-  for (int k = 0; k < 2; ++k) { diag->n_map[k] = dg.n_map[k]; diag->n_matches[k] = dg.n_matches[k]; copy_summary(dg.solve[k], &diag->solve[k]); }
-  std::memcpy(diag->pred_pose, dg.pred_pose, sizeof(dg.pred_pose));
+  copy_diag(dg, diag);
   return 0;
 }
 

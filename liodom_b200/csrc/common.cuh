@@ -198,7 +198,6 @@ __device__ __forceinline__ int lane_at(const DevBuffers& d, int pos) { return d.
 // list (d.lanes null, every single-lane entry point) position and lane coincide.
 struct LaneRange { int lane0, nlanes; };
 int launch_split(const DevBuffers& d, cudaStream_t s, LaneRange lr);
-int launch_extract(const DevBuffers& d, cudaStream_t s, LaneRange lr, bool want_keys);
 int launch_hash_build(const DevBuffers& d, cudaStream_t s, LaneRange lr);
 int launch_window_filter(const DevBuffers& d, cudaStream_t s, LaneRange lr);   // voxelgrid.cu; 0 launches when the filter is off
 int launch_hash_rebuild(const DevBuffers& d, cudaStream_t s, int lane);
@@ -213,7 +212,8 @@ int launch_lmap_gather(const DevBuffers& d, cudaStream_t s, int lane, float4* ou
 int extract_ring_cap(const DevParams& p);
 cudaError_t configure_extract_kernels();          // per device, from liodom_ctx_create
 size_t extract_smem_needed(const DevParams& p);   // largest dynamic shared memory request of k_extract / k_compact
-int launch_extract_rings(const DevBuffers& d, cudaStream_t s, LaneRange lr, int ring0, int nrings);
+// extraction = launch_extract_rings (rings [ring0, ring0 + nrings)) + launch_compact
+int launch_extract_rings(const DevBuffers& d, cudaStream_t s, LaneRange lr, int ring0, int nrings, bool want_keys);
 int launch_compact(const DevBuffers& d, cudaStream_t s, LaneRange lr);
 int launch_associate_shard(const DevBuffers& d, cudaStream_t s, int lane, int outer_it, int rank, int world);
 

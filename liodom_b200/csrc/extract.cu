@@ -739,27 +739,17 @@ size_t extract_smem_needed(const DevParams& p) {   // + 4 KB for the kernels' st
   return (a > b ? a : b) + 4096;
 }
 
-int launch_extract_rings(const DevBuffers& d, cudaStream_t s, LaneRange lr, int ring0, int nrings) {
+int launch_extract_rings(const DevBuffers& d, cudaStream_t s, LaneRange lr, int ring0, int nrings, bool want_keys) {
   const int ring_cap = extract_ring_cap(d.p);
   const size_t sm = extract_smem_bytes(d.p, ring_cap);
-  if (extract_long_rings(d.p, ring_cap)) k_extract<1024><<<dim3(nrings, lr.nlanes), 1024, sm, s>>>(d, lr.lane0, ring_cap, 0, ring0);
-  else k_extract<256><<<dim3(nrings, lr.nlanes), 256, sm, s>>>(d, lr.lane0, ring_cap, 0, ring0);
+  if (extract_long_rings(d.p, ring_cap)) k_extract<1024><<<dim3(nrings, lr.nlanes), 1024, sm, s>>>(d, lr.lane0, ring_cap, want_keys, ring0);
+  else k_extract<256><<<dim3(nrings, lr.nlanes), 256, sm, s>>>(d, lr.lane0, ring_cap, want_keys, ring0);
   return 1;
 }
 int launch_compact(const DevBuffers& d, cudaStream_t s, LaneRange lr) {
   const int LR = d.p.scan_lines * d.p.scan_regions;
   k_compact<<<lr.nlanes, 1024, (LR + 32) * sizeof(int), s>>>(d, lr.lane0);
   return 1;
-}
-
-int launch_extract(const DevBuffers& d, cudaStream_t s, LaneRange lr, bool want_keys) {
-  const int ring_cap = extract_ring_cap(d.p);
-  const size_t sm = extract_smem_bytes(d.p, ring_cap);
-  if (extract_long_rings(d.p, ring_cap)) k_extract<1024><<<dim3(d.p.scan_lines, lr.nlanes), 1024, sm, s>>>(d, lr.lane0, ring_cap, want_keys ? 1 : 0, 0);
-  else k_extract<256><<<dim3(d.p.scan_lines, lr.nlanes), 256, sm, s>>>(d, lr.lane0, ring_cap, want_keys ? 1 : 0, 0);
-  const int LR = d.p.scan_lines * d.p.scan_regions;
-  k_compact<<<lr.nlanes, 1024, (LR + 32) * sizeof(int), s>>>(d, lr.lane0);
-  return 2;
 }
 
 }  // namespace liodom

@@ -1329,8 +1329,8 @@ static int assoc_group_size(int edges_per_lane, int nlanes, int world) {
   return edges_in_flight <= 12 * 5632 ? 4 : 1;
 }
 
-static void launch_associate_any(const DevBuffers& d, cudaStream_t s, int lane0, int nlanes, int edges_per_lane, int outer_it, int force,
-                                 const double* pose_override, int rank, int world) {
+static int launch_associate_any(const DevBuffers& d, cudaStream_t s, int lane0, int nlanes, int edges_per_lane, int outer_it, int force,
+                                const double* pose_override, int rank, int world) {
   const int G = assoc_group_size(edges_per_lane, nlanes, world);
   const dim3 g((unsigned)(((long long)edges_per_lane * G + kAssocThreads - 1) / kAssocThreads), nlanes);
   if (G == 16) k_associate<16><<<g, kAssocThreads, 0, s>>>(d, lane0, outer_it, force, pose_override, rank, world);
@@ -1346,16 +1346,16 @@ static void launch_associate_any(const DevBuffers& d, cudaStream_t s, int lane0,
     if (pooled) k_associate_pool<<<g, kAssocThreads, 0, s>>>(d, lane0, outer_it, force, pose_override, rank, world);
     else k_associate<1><<<g, kAssocThreads, 0, s>>>(d, lane0, outer_it, force, pose_override, rank, world);
     k_line_gate<<<dim3((edges_per_lane + 127) / 128, nlanes), 128, 0, s>>>(d, lane0, outer_it, force, rank, world);
+    return 2;
   }
+  return 1;   // the G = 4 / 8 / 16 kernels gate in place
 }
 
 int launch_associate(const DevBuffers& d, cudaStream_t s, LaneRange lr, int outer_it, bool force, const double* pose_override) {
-  launch_associate_any(d, s, lr.lane0, lr.nlanes, d.p.Ecap, outer_it, force ? 1 : 0, pose_override, 0, 1);
-  return 2;
+  return launch_associate_any(d, s, lr.lane0, lr.nlanes, d.p.Ecap, outer_it, force ? 1 : 0, pose_override, 0, 1);
 }
 int launch_associate_shard(const DevBuffers& d, cudaStream_t s, int lane, int outer_it, int rank, int world) {
-  launch_associate_any(d, s, lane, 1, edge_share(d.p.Ecap, world), outer_it, 0, nullptr, rank, world);
-  return 2;
+  return launch_associate_any(d, s, lane, 1, edge_share(d.p.Ecap, world), outer_it, 0, nullptr, rank, world);
 }
 
 // ---------------------------------------------------------------------------------------
