@@ -250,9 +250,12 @@ __device__ __forceinline__ unsigned hash_cell(unsigned long long k) {
 // Edge-sharded mode (world > 1 ranks per lane): rank r associates and solves the Morton positions
 // [r * share, (r + 1) * share) of the lane's n edges.  A multiple of 32, so every rank starts on a warp boundary.
 __host__ __device__ __forceinline__ int edge_share(int n, int world) { return ((n + world - 1) / world + 31) & ~31; }
-// word of the occupancy filter holding cell (ix, iy, iz): 32 consecutive cells along x share a word
+// word of the occupancy filter holding cell (ix, iy, iz): 32 consecutive cells along x share a word (ixhi = ix >> 5).
+// The filter is indexed by the 16-bit coordinates of pack_cell, so cells that share a hash slot also share a filter
+// bit: the bit is published once per slot (by the point that creates it), and a cell aliasing an occupied one
+// 32.8 km away must read as occupied.  (ix >> 5) & 0x7FF == (ix & 0xFFFF) >> 5, and the bit, ix & 31, is unchanged.
 __device__ __forceinline__ unsigned bloom_word_index(int ixhi, int iy, int iz, unsigned bmask) {
-  unsigned h = (unsigned)ixhi * 0x9E3779B1u ^ (unsigned)iy * 0x85EBCA77u ^ (unsigned)iz * 0xC2B2AE3Du;
+  unsigned h = (unsigned)(ixhi & 0x7FF) * 0x9E3779B1u ^ (unsigned)(iy & 0xFFFF) * 0x85EBCA77u ^ (unsigned)(iz & 0xFFFF) * 0xC2B2AE3Du;
   h ^= h >> 15; h *= 0x2C1B3C6Du; h ^= h >> 12;
   return h & bmask;
 }

@@ -730,7 +730,12 @@ constexpr int kFbRadius = (int)(1.0f / kCell);   // cells covering the 1 m gate 
 constexpr int kFbSide = 2 * kFbRadius + 1;
 
 __device__ __forceinline__ float axis_gap(float q, int cell) {
-  const float lo = kCell * (float)cell, hi = lo + kCell;   // exact
+  // cell_of saturates: cell INT_MAX holds every point at >= 2^30 m and INT_MIN every point at <= -2^30 m, but their
+  // boxes below are [2^30, 2^30] and [-2^30, -2^30].  Clamping the query to [-2^30, 2^30] makes the gap to a saturated
+  // cell 0 for a query inside it, and only lowers the gap to any other cell (whose points lie between the clamp and
+  // the query's own side), so the bound stays below every point's distance.  |q| < 2^30: unchanged.
+  q = fminf(fmaxf(q, -0x1p30f), 0x1p30f);
+  const float lo = kCell * (float)cell, hi = lo + kCell;   // every point of a cell lies in [lo, hi] (lo is exact)
   // q < lo: lo - q (and q - hi < 0); q > hi: q - hi (and lo - q < 0); inside: both <= 0.  Branch-free; the compiler
   // turned the conditional form into divergent branches inside the neighbour loops.
   return fmaxf(fmaxf(__fsub_rn(lo, q), __fsub_rn(q, hi)), 0.0f);

@@ -114,6 +114,97 @@ def knn5_bruteforce(map_pts, q):
     return idx, d2o
 
 
+def cell_of(v):
+    """Voxel-hash cell of a coordinate: floor(v / 0.5), saturated to int32 like a float -> int conversion on the GPU."""
+    c = np.floor(np.asarray(v, np.float32) * np.float32(2.0)).astype(np.float64)
+    return np.clip(np.nan_to_num(c, nan=0.0), -2.0 ** 31, 2.0 ** 31 - 1).astype(np.int64)
+
+
+def knn5_gate(window, edges, pose, gate_margin=1e-9):
+    """src/laser_odometry.cc:300-344 restated: the edges transformed (double math, float store), the exact 5-NN over the
+    kNN target `window` under float32 L2_Simple ((dx*dx + dy*dy) + dz*dz, no FMA) in (d2, logical index) order, and the
+    line gate d2[4] < 1.0 and lambda2 > 3 lambda1.  Non-finite map points are skipped; a non-finite query has no
+    neighbours.
+
+    -> dict with
+      q_world [E,4]      the transformed edges;
+      knn_idx, knn_d2    the five best cut at d2 < 1.0 (-1 / +inf after the cut);
+      idx6, d2_6 [E,6]   the six best, uncut (-1 / +inf where the target has fewer finite points);
+      gate [E] uint8     bit 0: d2[4] < 1.0; bit 1: the line test, where decided;
+      decided [E] bool   the line test is decided: bit 0 clear, or |lambda2 - 3 lambda1| > gate_margin lambda2
+                         (eigenvalues of the double scatter, np.linalg.eigvalsh);
+      eig [E,3]          those eigenvalues (0 where bit 0 is clear);
+      tie [E] bool       equal d2 between neighbours 1..6 (inside the five, or between the 5th and the 6th);
+      fallback [E] bool  the 27-cell cube around the query's 0.5 m cell does not prove the list: fewer than five
+                         candidates there, or the 5th of them has d2 >= 0.25 (the search then walks the 5^3 cube)."""
+    w = np.asarray(window, np.float32).reshape(-1, 4)
+    with np.errstate(invalid="ignore"):
+        q = transform(np.asarray(edges, np.float32).reshape(-1, 4), pose)
+    E, M = len(q), len(w)
+    okm = np.isfinite(w[:, :3]).all(1)
+    okq = np.isfinite(q[:, :3]).all(1)
+    wc = np.stack([cell_of(w[:, a]) for a in range(3)], 1)
+    qc = np.stack([cell_of(q[:, a]) for a in range(3)], 1)
+    none = np.uint64(0xFFFFFFFFFFFFFFFF)
+    keys6 = np.full((E, 6), none, np.uint64)
+    cube5 = np.full(E, none, np.uint64)
+    rows = max(1, (1 << 22) // max(M, 1))
+    ids = np.arange(M, dtype=np.uint64)
+    for a in range(0, E, rows):
+        b = min(E, a + rows)
+        if M == 0:
+            break
+        with np.errstate(invalid="ignore", over="ignore"):
+            d = q[a:b, None, :3] - w[None, :, :3]
+            d2 = d[..., 0] * d[..., 0]
+            d2 = d2 + d[..., 1] * d[..., 1]
+            d2 = d2 + d[..., 2] * d[..., 2]
+        assert d2.dtype == np.float32
+        key = (d2.view(np.uint32).astype(np.uint64) << np.uint64(32)) | ids[None, :]
+        key[:, ~okm] = none
+        key[~okq[a:b]] = none
+        k = min(6, M)
+        part = np.partition(key, k - 1, axis=1)[:, :k] if M > k else key
+        keys6[a:b, :k] = np.sort(part, axis=1)[:, :k]
+        incube = (np.abs(qc[a:b, None, :] - wc[None, :, :]) <= 1).all(2)
+        ck = np.where(incube, key, none)
+        if M >= 5:
+            cube5[a:b] = np.partition(ck, 4, axis=1)[:, 4] if M > 5 else np.sort(ck, axis=1)[:, 4]
+    have = keys6 != none
+    idx6 = np.where(have, (keys6 & np.uint64(0xFFFFFFFF)).astype(np.int64), -1).astype(np.int32)
+    d2_6 = np.where(have, (keys6 >> np.uint64(32)).astype(np.uint32), np.uint32(0x7F800000)).view(np.float32)
+    d2_6 = d2_6.reshape(E, 6)
+    keep = have[:, :5] & (d2_6[:, :5] < np.float32(1.0))
+    knn_idx = np.where(keep, idx6[:, :5], -1).astype(np.int32)
+    knn_d2 = np.where(keep, d2_6[:, :5], np.float32(np.inf)).astype(np.float32)
+    tie = (have[:, 1:] & (d2_6[:, 1:] == d2_6[:, :-1])).any(1)
+    cube_d2 = np.where(cube5 != none, (cube5 >> np.uint64(32)).astype(np.uint32), np.uint32(0x7F800000)).view(np.float32)
+    fallback = okq & (cube_d2 >= np.float32(0.25))
+
+    gate = np.zeros(E, np.uint8)
+    decided = np.ones(E, bool)
+    eig = np.zeros((E, 3))
+    sel = np.nonzero(keep[:, 4])[0]
+    gate[sel] = 1
+    if len(sel):
+        nn = w[idx6[sel, :5], :3].astype(np.float64)              # [n,5,3], neighbour order
+        m = nn[:, 0]
+        for r in range(1, 5):
+            m = m + nn[:, r]
+        m = m / 5.0
+        C = np.zeros((len(sel), 3, 3))
+        for r in range(5):
+            dv = nn[:, r] - m
+            C = C + dv[:, :, None] * dv[:, None, :]
+        ev = np.linalg.eigvalsh(C)
+        eig[sel] = ev
+        dd = ev[:, 2] - 3.0 * ev[:, 1]
+        decided[sel] = np.abs(dd) > gate_margin * ev[:, 2]
+        gate[sel] |= np.where(decided[sel] & (dd > 0), 2, 0).astype(np.uint8)
+    return dict(q_world=q, knn_idx=knn_idx, knn_d2=knn_d2, idx6=idx6, d2_6=d2_6, gate=gate, decided=decided, eig=eig,
+                tie=tie, fallback=fallback)
+
+
 def quat_rotate(q, v):
     """Eigen unit-quaternion * vector, q = (x,y,z,w)."""
     qv, w = np.asarray(q[:3], float), float(q[3])

@@ -36,8 +36,9 @@ def _oracle_run(seed):
     return _ORACLE[seed]
 
 
-def _run_batch(batch, mode):
-    """mode: 'host_packed' (one buffer, scans back to back), 'host_lanes' (separate arrays), 'device'."""
+def _run_batch(batch, mode, trace=None):
+    """mode: 'host_packed' (one buffer, scans back to back), 'host_lanes' (separate arrays), 'device'.  `trace`, when
+    given, receives every frame's poses of all lanes."""
     seqs = [get_sequence("hdl64", 1000 + k, N_FRAMES)[0] for k in range(N_SEEDS)]
     ctx = api.Context(prev_frames=PREV, max_points=131072, batch=batch)
     worst = [0.0, 0.0]
@@ -60,6 +61,8 @@ def _run_batch(batch, mode):
             # every lane must read its own addresses only when timing matters; for parity, sharing is fine
             ctx.scan_batch_ptrs([dev[l % N_SEEDS][f].data_ptr() for l in range(batch)], cnts, 16, on_device=True)
         poses, ne = ctx.results()
+        if trace is not None:
+            trace.append(np.array(poses, copy=True))
         for l in range(batch):
             oposes, one = _oracle_run(1000 + l % N_SEEDS)
             assert ne[l] == one[f], "lane %d frame %d: %d edges, oracle %d" % (l, f, ne[l], one[f])
@@ -88,13 +91,22 @@ def test_batch128_lane_groups(cuda_lib, groups, monkeypatch):
     print("batch 128, %s lane groups: worst pose error %.3g m %.3g rad" % (groups, w[0], w[1]))
 
 
+_POOL_POSES = {}
+
+
 @pytest.mark.parametrize("pool", ["0", "1"])
 def test_batch128_warp_pooled_association(cuda_lib, pool, monkeypatch):
     """LIODOM_ASSOC_POOL=0 / 1: the thread-per-edge kernel in both outer iterations / the warp-pooled one in both (the
-    default is thread-per-edge first, pooled and seeded second: every other test of this file).  Same poses."""
+    default is thread-per-edge first, pooled and seeded second: every other test of this file).  Same poses, bit for
+    bit: both kernels claim the same five neighbours in the same order, and the gate and the solve are shared."""
     monkeypatch.setenv("LIODOM_ASSOC_POOL", pool)
-    w = _run_batch(128, "device")
+    trace = []
+    w = _run_batch(128, "device", trace)
+    _POOL_POSES[pool] = np.stack(trace)
     print("batch 128, LIODOM_ASSOC_POOL=%s: worst pose error %.3g m %.3g rad" % (pool, w[0], w[1]))
+    other = _POOL_POSES.get("1" if pool == "0" else "0")
+    if other is not None:
+        assert np.array_equal(_POOL_POSES[pool].view(np.uint64), other.view(np.uint64))
 
 
 @pytest.mark.parametrize("name", ["c2_ouster", "c3_stress"])
